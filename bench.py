@@ -5,6 +5,7 @@ Metric (BASELINE.json): kNN queries/s, k = 16, 10 M-point clouds, at 1/2/4/8 B20
 
   python bench.py --gpus N --steps K --warmup W          (N > 1: launched under torch.distributed.run)
   python bench.py --impl reference ...                   (the CPU path on the box's host cores, rank 0 only)
+  python bench.py ... --dump-outputs DIR                 (also writes a fixed sample of the last timed step's result rows to DIR/*.npy)
 
 One "step" = one pass of the hot path over one batch: pcc_knn (query cell keys -> radix sort -> fused kNN kernel)
 for ONE set of Q = 10 M query points against the 10 M-point indexed reference cloud, everything resident in HBM.
@@ -32,6 +33,8 @@ sys.path.insert(0, ROOT)
 METRIC = "knn_queries_per_s_k16_10M"
 UNIT = "queries/s"
 K = 16
+DUMP_BYTES = 64_000_000
+DUMP_SEED = 20240601
 
 
 def workload_config(args, world):
@@ -106,6 +109,23 @@ def make_clouds(args, rank):
     return ref, qry
 
 
+def dump_rows(n: int, k: int):
+    """Positions of the result rows --dump-outputs writes: all n when they fit in DUMP_BYTES, else a fixed seeded sample
+    (ascending).  A row costs k float64 indices, k float32 squared distances and its float64 query row number."""
+    fit = max(1, (DUMP_BYTES - 4096) // (12 * k + 8))
+    if n <= fit:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, fit, replace=False))
+
+
+def dump_outputs(path: str, query_rows, idx, d2):
+    """Result rows of the timed path as <path>/<name>.npy; indices as float64, which holds every int32 exactly."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("query_rows", np.asarray(query_rows, np.float64)), ("knn_indices", np.asarray(idx, np.float64)),
+                    ("knn_sqr_distances", np.asarray(d2, np.float32))):
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def host_threads() -> int:
     """Threads the CPU arm uses: every core this process may run on.  Set explicitly on each call -- torch.distributed.run
     exports OMP_NUM_THREADS=1, which made the round-1 reference arm single-threaded at N >= 2."""
@@ -147,10 +167,14 @@ def run_reference(args):
     total = args.warmup + args.steps
     times = []
     for s in range(total):
-        q = qry[(s * sample) % max(args.nq - sample, 1):][:sample]
+        start = (s * sample) % max(args.nq - sample, 1)
+        q = qry[start:][:sample]
         t0 = time.perf_counter()
-        tree.knn(q, args.k, threads=cores)
+        idx, d2, _ = tree.knn(q, args.k, threads=cores)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        pick = dump_rows(len(q), args.k)
+        dump_outputs(args.dump_outputs, start + pick, idx[pick], d2[pick])
     t = sum(times[args.warmup:])
     value = sample * args.steps / t
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -261,6 +285,15 @@ def run_ours(args):
 
     ms = _events_ms(step, args.steps, barrier, world, dist, torch)
     launches = launch_count() - l0
+    if args.dump_outputs:                    # `out` is the last timed step's result; N > 1: each rank holds its shard, gathered into query order
+        ti, td = out[0], out[1]
+        if world > 1:
+            ti, td = s.gather(ti, drows, args.nq), s.gather(td, drows, args.nq)
+        if rank == 0:
+            pick = dump_rows(args.nq, args.k)
+            sel = torch.from_numpy(pick).to(dev)
+            dump_outputs(args.dump_outputs, pick, ti[sel].cpu().numpy(), td[sel].cpu().numpy())
+        del ti, td
     rank_ms = None
     if world > 1:                # per-rank time of the same steps (load balance of the shards), gathered for the JSON line
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -472,7 +505,11 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="skip the ICP 10 M vs 10 M arm (BASELINE configs[3])")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling comparison steps at N > 1")
     ap.add_argument("--shard-block", type=int, default=8192, help="queries per block of the cell order dealt round-robin to the ranks (0 = one contiguous range per rank)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's result rows (all of them, or a fixed seeded "
+                                                             "sample within 64 MB) as DIR/query_rows.npy, DIR/knn_indices.npy and DIR/knn_sqr_distances.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -2,15 +2,31 @@
 
 The reference has no tests or golden vectors for this path (SURVEY.md section 4) and PCL/FLANN are not
 installable here, so the pins are: (1) committed golden vectors produced by OpenCV's bundled
-FLANN KDTreeSingleIndex (tests/golden/make_golden.py), (2) the same library called live when
-cv2 is importable, (3) scipy cKDTree at set level, (4) hand-derived known answers.
+FLANN KDTreeSingleIndex (tests/golden/make_golden.py), (2) the same library's answers on larger
+and 32-D inputs, recorded by the same script, (3) scipy cKDTree at set level, (4) hand-derived
+known answers.
 """
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
 import oracle
 from conftest import bits
 from pointcloudcomparator_b200 import synth
+
+
+@pytest.fixture(scope="module")
+def flann():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "opencv_flann_pins.npz"))
+
+
+def _recorded(flann, name, ref, qry):
+    """(idx, d2) of OpenCV's FLANN KDTreeSingleIndex (leaf 15, exact, sorted) on these inputs, as tests/golden/make_golden.py recorded them."""
+    ref, qry = np.ascontiguousarray(ref, np.float32), np.ascontiguousarray(qry, np.float32)
+    assert str(flann[f"{name}_inputs_sha256"]) == hashlib.sha256(ref.tobytes() + qry.tobytes()).hexdigest(), f"{name}: inputs differ from the recorded ones"
+    return flann[f"{name}_idx"], flann[f"{name}_d2"]
 
 
 def test_golden_knn(golden):
@@ -32,24 +48,20 @@ def test_golden_radius(golden):
         assert np.array_equal(bits(d2), bits(golden["rad_d2"]))
 
 
-def test_live_opencv_flann():
-    cv2 = pytest.importorskip("cv2")
+def test_recorded_opencv_flann_knn(flann):
     ref = synth.room(60000, 1001)
-    qry = synth.sweep_queries(ref, 3000, seed=9)
-    fl = cv2.flann_Index(ref, dict(algorithm=4, leaf_max_size=15))
-    ci, cd = fl.knnSearch(qry, 16, params=dict(checks=-1, eps=0.0, sorted=True))
+    qry = synth.sweep_queries(ref, 3000, seed=9)[::3]
+    ci, cd = _recorded(flann, "room60k_knn16", ref, qry)
     ti, td, _ = oracle.KdTree(ref).knn(qry, 16)
     assert np.array_equal(ci, ti) and np.array_equal(bits(cd), bits(td))
 
 
-def test_lattice_ties_distance_multiset_matches_flann():
+def test_lattice_ties_distance_multiset_matches_flann(flann):
     """FLANN keeps visit order among equal d2; the canonical order is (d2, idx).  Distances agree always."""
-    cv2 = pytest.importorskip("cv2")
     g = np.arange(12, dtype=np.float32)
     ref = np.stack(np.meshgrid(g, g, g, indexing="ij"), -1).reshape(-1, 3)
     qry = np.ascontiguousarray(ref[::7])
-    fl = cv2.flann_Index(ref, dict(algorithm=4, leaf_max_size=15))
-    _, cd = fl.knnSearch(qry, 8, params=dict(checks=-1, eps=0.0, sorted=True))
+    _, cd = _recorded(flann, "lattice_knn8", ref, qry)
     ti, td, _ = oracle.KdTree(ref).knn(qry, 8)
     bi, bd, _ = oracle.brute_knn(ref, qry, 8)
     assert np.array_equal(bits(cd), bits(td))
@@ -189,13 +201,11 @@ def test_voxel_grid_known_answers():
     assert len(np.unique(vox, axis=0)) >= 0.999 * o.shape[0]      # every centroid stays inside its own voxel (up to fp32 rounding on faces)
 
 
-def test_descriptor_nn_matches_opencv_flann_32d():
-    cv2 = pytest.importorskip("cv2")
+def test_descriptor_nn_matches_opencv_flann_32d(flann):
     rng = np.random.default_rng(3)
     ref = rng.random((700, 32), dtype=np.float32) * 0.3
     qry = (ref[rng.integers(0, 700, 400)] + rng.normal(0, 0.02, (400, 32))).astype(np.float32)
-    fl = cv2.flann_Index(ref, dict(algorithm=4, leaf_max_size=15))          # same index family KdTreeFLANN<Histogram<32>> builds
-    ci, cd = fl.knnSearch(qry, 1, params=dict(checks=-1, eps=0.0, sorted=True))
+    ci, cd = _recorded(flann, "desc32_nn", ref, qry)                       # same index family KdTreeFLANN<Histogram<32>> builds
     oi, od = oracle.descriptor_nn(ref, qry)
     # OpenCV's FLANN uses the 4-way unrolled cvflann::L2 functor (sums four squared differences per step); PCL's KdTreeFLANN
     # uses L2_Simple (one dimension at a time), which the oracle restates.  Same neighbours, distances equal to a few ulp.
@@ -491,16 +501,14 @@ def test_icp_vs_numpy_loop():
     assert np.isclose(r["fitness"], fit, rtol=2e-3)
 
 
-def test_descriptor_nn_three_dims_matches_flann_on_first_three_bins():
+def test_descriptor_nn_three_dims_matches_flann_on_first_three_bins(flann):
     """PCL 1.7's DefaultPointRepresentation clamps an unregistered point type to its first 3 floats, so the reference's
     KdTreeFLANN<Histogram<32>> (src/comparator.cpp:564-577) is a 3-D tree over bins 0..2: the oracle's dims = 3 mode against a
     FLANN KDTreeSingleIndex built on exactly those columns."""
-    cv2 = pytest.importorskip("cv2")
     rng = np.random.default_rng(8)
     ref = rng.random((900, 32), dtype=np.float32) * 0.3
     qry = (ref[rng.integers(0, 900, 500)] + rng.normal(0, 0.02, (500, 32))).astype(np.float32)
-    fl = cv2.flann_Index(np.ascontiguousarray(ref[:, :3]), dict(algorithm=4, leaf_max_size=15))
-    ci, cd = fl.knnSearch(np.ascontiguousarray(qry[:, :3]), 1, params=dict(checks=-1, eps=0.0, sorted=True))
+    ci, cd = _recorded(flann, "desc3_nn", ref[:, :3], qry[:, :3])
     oi, od = oracle.descriptor_nn(ref, qry, dims=3)
     assert np.array_equal(ci[:, 0], oi) and np.allclose(cd[:, 0], od, rtol=1e-6, atol=0)
     o32, _ = oracle.descriptor_nn(ref, qry)
