@@ -16,6 +16,8 @@
 //   pcc::findPointNeighbours         <- RegionGrowing(RGB)::findPointNeighbours (src/segmentation.cpp:271,190)
 //   pcc::VoxelGrid                   <- pcl::VoxelGrid                   (src/segmentation.cpp:69-74,223-228)
 //   pcc::RegionGrowing               <- pcl::RegionGrowing               (src/segmentation.cpp:249-271)
+//   pcc::IntensityGradientEstimation <- pcl::IntensityGradientEstimation (src/comparator.cpp:649-656)
+//   pcc::RIFTEstimation              <- pcl::RIFTEstimation              (src/comparator.cpp:659-673)
 // There is no CPU fallback: a failing CUDA call throws pcc::Error.
 #ifndef PCC_GRID_SEARCH_HPP_
 #define PCC_GRID_SEARCH_HPP_
@@ -461,6 +463,81 @@ class RegionGrowingRGB {
     int rgba_off_, table_k_ = 100, grow_k_ = 30;
     int64_t min_size_ = 1, max_size_ = std::numeric_limits<int>::max();
     float distance_ = 10.f, point_color_ = 1225.f, region_color_ = 10.f;          // PCL 1.7 constructor defaults
+};
+
+// PCL 1.7 PointXYZRGBtoXYZI (src/comparator.cpp:597): 0.299f r + 0.587f g + 0.114f b, left to right in fp32.
+inline float rgbToIntensity(std::uint8_t r, std::uint8_t g, std::uint8_t b) {
+    volatile float t = 0.299f * (float)r;          // volatile: no contraction into an FMA whatever the caller's flags
+    t = t + 0.587f * (float)g;
+    return t + 0.114f * (float)b;
+}
+
+struct IntensityGradient { float gradient_x, gradient_y, gradient_z, _pad; };
+struct Histogram32 { float histogram[32]; };
+
+// pcl::IntensityGradientEstimation<PointT, Normal, IntensityGradient>::compute with setRadiusSearch(r) over the tree's input
+// cloud (the reference's surface): one fused GPU call (pcc_intensity_gradient).  Intensities are one float per input point
+// (rgbToIntensity for colour clouds); normals as pcc::NormalEstimation fills them.  NaN gradients with < 3 neighbours.
+template <typename PointT>
+class IntensityGradientEstimation {
+  public:
+    void setSearchMethod(const typename search::GridSearch<PointT>::Ptr &tree) { tree_ = tree; }
+    void setInputCloud(const typename search::GridSearch<PointT>::PointCloudConstPtr &cloud) { input_ = cloud; }
+    void setInputNormals(const std::vector<Normal> *normals) { normals_ = normals; }
+    void setInputIntensities(const std::vector<float> *intensity) { intensity_ = intensity; }
+    void setRadiusSearch(double r) { radius_ = r; }
+    void compute(std::vector<IntensityGradient> &out) {
+        if (!input_ || !normals_ || !intensity_ || normals_->size() != input_->points.size() || intensity_->size() != input_->points.size())
+            throw Error("IntensityGradientEstimation: cloud, normals and intensities must be set and of equal size");
+        if (!tree_) tree_.reset(new search::GridSearch<PointT>());
+        tree_->setCellHint((float)radius_);
+        if (tree_->getInputCloud() != input_) tree_->setInputCloud(input_);
+        const size_t n = input_->points.size();
+        std::vector<float> nrm(n * 4), flat(n * 4);
+        for (size_t i = 0; i < n; ++i) { const Normal &m = (*normals_)[i]; nrm[4 * i] = m.normal_x; nrm[4 * i + 1] = m.normal_y; nrm[4 * i + 2] = m.normal_z; nrm[4 * i + 3] = m.curvature; }
+        if (n) check(pcc_intensity_gradient(tree_->handle(), nullptr, 0, (int)sizeof(PointT), radius_, intensity_->data(), nrm.data(), flat.data(), PCC_HOST, nullptr));
+        out.resize(n);
+        for (size_t i = 0; i < n; ++i) { out[i].gradient_x = flat[4 * i]; out[i].gradient_y = flat[4 * i + 1]; out[i].gradient_z = flat[4 * i + 2]; out[i]._pad = 0.f; }
+    }
+  private:
+    typename search::GridSearch<PointT>::Ptr tree_;
+    typename search::GridSearch<PointT>::PointCloudConstPtr input_;
+    const std::vector<Normal> *normals_ = nullptr;
+    const std::vector<float> *intensity_ = nullptr;
+    double radius_ = 0;
+};
+
+// pcl::RIFTEstimation<PointT, IntensityGradient, Histogram<32>>::compute over the tree's input cloud (pcc_rift).  Bins beyond
+// nd * ng stay 0; a point without neighbours gets a NaN histogram.  Order: histogram[g * nd + d], as PCL copies it out.
+template <typename PointT>
+class RIFTEstimation {
+  public:
+    void setSearchMethod(const typename search::GridSearch<PointT>::Ptr &tree) { tree_ = tree; }
+    void setInputCloud(const typename search::GridSearch<PointT>::PointCloudConstPtr &cloud) { input_ = cloud; }
+    void setInputGradient(const std::vector<IntensityGradient> *gradient) { gradient_ = gradient; }
+    void setRadiusSearch(double r) { radius_ = r; }
+    void setNrDistanceBins(int n) { nd_ = n; }
+    void setNrGradientBins(int n) { ng_ = n; }
+    void compute(std::vector<Histogram32> &out) {
+        if (!input_ || !gradient_ || gradient_->size() != input_->points.size())
+            throw Error("RIFTEstimation: the gradient cloud must be set and of the input cloud's size");
+        if (nd_ * ng_ > 32) throw Error("RIFTEstimation: nr_distance_bins * nr_gradient_bins must be <= 32 (Histogram<32>)");
+        if (!tree_) tree_.reset(new search::GridSearch<PointT>());
+        tree_->setCellHint((float)radius_);
+        if (tree_->getInputCloud() != input_) tree_->setInputCloud(input_);
+        const size_t n = input_->points.size();
+        const int nb = nd_ * ng_;
+        std::vector<float> flat(n * (size_t)nb);
+        if (n) check(pcc_rift(tree_->handle(), nullptr, 0, (int)sizeof(PointT), radius_, reinterpret_cast<const float *>(gradient_->data()), nd_, ng_, flat.data(), PCC_HOST, nullptr));
+        out.assign(n, Histogram32());
+        for (size_t i = 0; i < n; ++i) for (int k = 0; k < 32; ++k) out[i].histogram[k] = k < nb ? flat[i * nb + k] : 0.f;
+    }
+  private:
+    typename search::GridSearch<PointT>::Ptr tree_;
+    typename search::GridSearch<PointT>::PointCloudConstPtr input_;
+    const std::vector<IntensityGradient> *gradient_ = nullptr;
+    double radius_ = 0;
+    int nd_ = 4, ng_ = 8;
 };
 
 // matchRIFTFeaturesKnn (src/comparator.cpp:560-588): KdTreeFLANN<Histogram<32>> over descriptors1, nearestKSearch(k = 1) for every

@@ -95,6 +95,21 @@ int pcc_normals_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
 int pcc_normals_radius(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float viewpoint[3],
                        float *out, int mem, void *stream);
 
+/* IntensityGradientEstimation::computeFeature (src/comparator.cpp:649-656, r = 0.03) [up]. intensity[n_input]: one float per INPUT
+ * row of the indexed cloud (original order). normals4[rows*4]: the query's (nx, ny, nz, curvature) as pcc_normals_* writes them,
+ * rows = nq, or n_input when q == NULL. out[rows*4] = gx, gy, gz, 0; NaN with < 3 neighbours and for skipped (non-finite) rows.
+ * Per query over its (d2, idx)-sorted radius row: fp32 centroid and mean intensity (true divisions), A = sum (p-c)(p-c)^T and
+ * b = sum (p-c)(I-mean) in row order (non-finite intensities skipped), x = Eigen 3.3 colPivHouseholderQr(A).solve(b) -- rank-
+ * deficient A (planar neighbourhoods) solves over the nonzero pivots only -- and gradient = (I - n n^T) x. */
+int pcc_intensity_gradient(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *intensity,
+                           const float *normals4, float *out, int mem, void *stream);
+/* RIFTEstimation::computeFeature (src/comparator.cpp:659-673, r = 0.05, 4 x 8 bins) [up]. gradient4[n_input*4] per INPUT row of the
+ * indexed cloud. out[rows * nd*ng] in PCL's histogram order; NaN row without neighbours. nd*ng <= 32 (Histogram<32>), else PCC_ERR_INVALID.
+ * PCL's histogram order is gradient bin outer, distance bin inner: out[row*nd*ng + g*nd + d].  The query point is both the search
+ * centre and p0; each histogram is normalised to unit Frobenius norm (an all-zero one stays zero). */
+int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *gradient4,
+             int n_distance_bins, int n_gradient_bins, float *out, int mem, void *stream);
+
 /* CorrespondenceEstimation::determineCorrespondences + the sums TransformationEstimationSVD needs
  * (src/comparator.cpp:1091-1096) [up].  Each source point is first moved by the row-major 4x4 `T_apply`
  * (IterativeClosestPoint::transformCloud arithmetic; NULL = identity) IN PLACE when `src_inout` is device

@@ -423,4 +423,129 @@ __device__ __forceinline__ void accu_add(float *a, float x, float y, float z) {
     a[0] += x * x; a[1] += x * y; a[2] += x * z; a[3] += y * y; a[4] += y * z; a[5] += z * z; a[6] += x; a[7] += y; a[8] += z;
 }
 
+// Eigen's completely unrolled reduction of a fixed-size 3-vector (norm, dot, 3x3 * vector): a0 + (a1 + a2)
+__device__ __forceinline__ float sum3(float a0, float a1, float a2) { return a0 + (a1 + a2); }
+
+// x = A.colPivHouseholderQr().solve(b) for a 3x3 fp32 system, Eigen 3.3's ColPivHouseholderQR restated (DESIGN.md section 2):
+// largest-remaining-norm pivot (first on ties) with the LAPACK norm downdate, makeHouseholderInPlace, rank = pivots before the
+// first column whose squared norm falls below (max norm * eps)^2 / 3 * (3 - k), back substitution over those pivots, zeros for
+// the rest.  a is column-major (a[r + 3c]); with -fmad=false every operation below is one correctly rounded fp32 op.
+__device__ __forceinline__ void colpiv_qr_solve(float a[9], const float b[3], float x[3]) {
+    const float eps = 1.1920929e-07f;
+    float hc[3], nu[3], nd[3];
+    int perm[3] = {0, 1, 2};
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { nd[k] = sqrtf(sum3(a[3 * k] * a[3 * k], a[3 * k + 1] * a[3 * k + 1], a[3 * k + 2] * a[3 * k + 2])); nu[k] = nd[k]; }
+    float mx = nu[0];
+    if (nu[1] > mx) mx = nu[1];
+    if (nu[2] > mx) mx = nu[2];
+    const float te = mx * eps;
+    const float threshold_helper = __fdiv_rn(te * te, 3.0f);
+    const float norm_downdate_threshold = sqrtf(eps);
+    int np = 3;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        int bi = k;
+#pragma unroll
+        for (int j = k + 1; j < 3; ++j) if (nu[j] > nu[bi]) bi = j;
+        const float bsq = nu[bi] * nu[bi];
+        if (np == 3 && bsq < threshold_helper * (float)(3 - k)) np = k;
+        if (bi != k) {        // bi is a run-time index: swap through selects so everything stays in registers
+#pragma unroll
+            for (int j = k + 1; j < 3; ++j) {
+                if (j == bi) {
+#pragma unroll
+                    for (int r = 0; r < 3; ++r) { const float t = a[r + 3 * k]; a[r + 3 * k] = a[r + 3 * j]; a[r + 3 * j] = t; }
+                    float t = nu[k]; nu[k] = nu[j]; nu[j] = t;
+                    t = nd[k]; nd[k] = nd[j]; nd[j] = t;
+                    const int ti = perm[k]; perm[k] = perm[j]; perm[j] = ti;
+                }
+            }
+        }
+        const float c0 = a[k + 3 * k];
+        float tail_sq = 0.f;
+#pragma unroll
+        for (int r = k + 1; r < 3; ++r) tail_sq = (r == k + 1) ? a[r + 3 * k] * a[r + 3 * k] : tail_sq + a[r + 3 * k] * a[r + 3 * k];
+        float tau, beta;
+        if (tail_sq <= 1.17549435e-38f) {
+            tau = 0.f; beta = c0;
+#pragma unroll
+            for (int r = k + 1; r < 3; ++r) a[r + 3 * k] = 0.f;
+        } else {
+            beta = sqrtf(c0 * c0 + tail_sq);
+            if (c0 >= 0.f) beta = -beta;
+            const float den = c0 - beta;
+#pragma unroll
+            for (int r = k + 1; r < 3; ++r) a[r + 3 * k] = __fdiv_rn(a[r + 3 * k], den);
+            tau = __fdiv_rn(beta - c0, beta);
+        }
+        hc[k] = tau;
+        a[k + 3 * k] = beta;
+        if (tau != 0.f) {
+#pragma unroll
+            for (int j = k + 1; j < 3; ++j) {
+                float t = 0.f;
+#pragma unroll
+                for (int r = k + 1; r < 3; ++r) t += a[r + 3 * k] * a[r + 3 * j];
+                t = t + a[k + 3 * j];
+                a[k + 3 * j] = a[k + 3 * j] - tau * t;
+#pragma unroll
+                for (int r = k + 1; r < 3; ++r) a[r + 3 * j] = a[r + 3 * j] - t * (tau * a[r + 3 * k]);
+            }
+        }
+#pragma unroll
+        for (int j = k + 1; j < 3; ++j) {
+            if (nu[j] != 0.f) {
+                float t = __fdiv_rn(fabsf(a[k + 3 * j]), nu[j]);
+                t = (1.f + t) * (1.f - t);
+                t = t < 0.f ? 0.f : t;
+                const float q = __fdiv_rn(nu[j], nd[j]);
+                const float t2 = t * (q * q);
+                if (t2 <= norm_downdate_threshold) {
+                    float s = 0.f;
+#pragma unroll
+                    for (int r = k + 1; r < 3; ++r) s = (r == k + 1) ? a[r + 3 * j] * a[r + 3 * j] : s + a[r + 3 * j] * a[r + 3 * j];
+                    nd[j] = sqrtf(s);
+                    nu[j] = nd[j];
+                } else {
+                    nu[j] *= sqrtf(t);
+                }
+            }
+        }
+    }
+    x[0] = x[1] = x[2] = 0.f;
+    if (np == 0) return;
+    float c[3] = {b[0], b[1], b[2]};
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        if (k < np) {
+            if (k == 2) { c[2] = c[2] * (1.f - hc[2]); }
+            else if (hc[k] != 0.f) {
+                float t = a[k + 1 + 3 * k] * c[k + 1];
+#pragma unroll
+                for (int r = k + 2; r < 3; ++r) t = t + a[r + 3 * k] * c[r];
+                t = t + c[k];
+                c[k] = c[k] - hc[k] * t;
+#pragma unroll
+                for (int r = k + 1; r < 3; ++r) c[r] = c[r] - t * (hc[k] * a[r + 3 * k]);
+            }
+        }
+    }
+#pragma unroll
+    for (int i = 2; i >= 0; --i) {
+        if (i < np && c[i] != 0.f) {
+            c[i] = __fdiv_rn(c[i], a[i + 3 * i]);
+#pragma unroll
+            for (int s = 0; s < i; ++s) c[s] = c[s] - c[i] * a[s + 3 * i];
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        if (i < np) {
+#pragma unroll
+            for (int j = 0; j < 3; ++j) if (perm[i] == j) x[j] = c[i];
+        }
+    }
+}
+
 }  // namespace pcc

@@ -330,6 +330,160 @@ __global__ void __launch_bounds__(128) normals_rows_kernel(Grid g, QueryView v, 
     out[row] = normal_from_accu(a, (int)min((int64_t)INT_MAX, e - b), x, y, z, vx, vy, vz);
 }
 
+__device__ __forceinline__ int64_t rows_query(const Grid &g, const QueryView &v, int64_t t, float &x, float &y, float &z) {
+    if (v.self) { float4 p = __ldg(g.pts + t); x = p.x; y = p.y; z = p.z; return __float_as_int(p.w); }
+    uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t; float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; return qi;
+}
+
+// IntensityGradientEstimation(radius), is_dense branch: centroid and mean intensity over the sorted row, then
+// A = sum (p-c)(p-c)^T (upper triangle) and b = sum (p-c)(I-mean) in row order, x = colPivHouseholderQr(A).solve(b),
+// gradient = (I - n n^T) x.  Intensity is read by original index, the normal by the query's row.
+__global__ void __launch_bounds__(128) gradient_rows_kernel(Grid g, QueryView v, const int64_t *__restrict__ offsets, const nkey_t *__restrict__ keys,
+                                                            const uint32_t *__restrict__ inv_pos, const float *__restrict__ intensity,
+                                                            const float4 *__restrict__ normals, float4 *__restrict__ out) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= v.nq) return;
+    float qx, qy, qz;
+    const int64_t row = rows_query(g, v, t, qx, qy, qz);
+    const int64_t b = offsets[row], e = offsets[row + 1];
+    const float qnan = CUDART_NAN_F;
+    if (e - b < 3) { out[row] = make_float4(qnan, qnan, qnan, 0.f); return; }
+    float cx = 0.f, cy = 0.f, cz = 0.f, mi = 0.f;
+    for (int64_t j = b; j < e; ++j) {
+        const uint32_t id = (uint32_t)keys[j];
+        const float4 p = __ldg(g.pts + __ldg(inv_pos + id));
+        cx += p.x; cy += p.y; cz += p.z;
+        mi += __ldg(intensity + id);
+    }
+    const float fn = (float)(e - b);
+    cx = __fdiv_rn(cx, fn); cy = __fdiv_rn(cy, fn); cz = __fdiv_rn(cz, fn); mi = __fdiv_rn(mi, fn);
+    float a00 = 0.f, a01 = 0.f, a02 = 0.f, a11 = 0.f, a12 = 0.f, a22 = 0.f, b0 = 0.f, b1 = 0.f, b2 = 0.f;
+    for (int64_t j = b; j < e; ++j) {
+        const uint32_t id = (uint32_t)keys[j];
+        const float4 p = __ldg(g.pts + __ldg(inv_pos + id));
+        const float in = __ldg(intensity + id);
+        if (!isfinite(in)) continue;                 // indexed points are finite; a non-finite intensity is skipped like PCL
+        const float x = p.x - cx, y = p.y - cy, z = p.z - cz, w = in - mi;
+        a00 += x * x; a01 += x * y; a02 += x * z;
+        a11 += y * y; a12 += y * z;
+        a22 += z * z;
+        b0 += x * w; b1 += y * w; b2 += z * w;
+    }
+    float A[9] = {a00, a01, a02, a01, a11, a12, a02, a12, a22};
+    const float rhs[3] = {b0, b1, b2};
+    float xs[3];
+    colpiv_qr_solve(A, rhs, xs);
+    const float4 n = __ldg(normals + row);
+    const float nn[3] = {n.x, n.y, n.z};
+    float gr[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const float m0 = (r == 0 ? 1.f : 0.f) - nn[r] * nn[0];
+        const float m1 = (r == 1 ? 1.f : 0.f) - nn[r] * nn[1];
+        const float m2 = (r == 2 ? 1.f : 0.f) - nn[r] * nn[2];
+        gr[r] = sum3(m0 * xs[0], m1 * xs[1], m2 * xs[2]);
+    }
+    out[row] = make_float4(gr[0], gr[1], gr[2], 0.f);
+}
+
+// Eigen 3.3's SSE squared-norm reduction (MatrixXf::normalize) over the first nb of 32 register-resident bins: packets of 4 in
+// two accumulators, predux (l0 + l2) + (l1 + l3), then the scalar tail.  Loops are unrolled over all 32 slots so h stays in registers.
+__device__ __forceinline__ float rift_sq_norm(const float (&h)[32], int nb) {
+    if (nb < 4) {
+        float s = h[0] * h[0];
+#pragma unroll
+        for (int i = 1; i < 3; ++i) if (i < nb) s = s + h[i] * h[i];
+        return s;
+    }
+    const int aligned = nb & ~3, aligned2 = nb & ~7;
+    float r0[4], r1[4];
+#pragma unroll
+    for (int l = 0; l < 4; ++l) r0[l] = h[l] * h[l];
+    if (aligned > 4) {
+#pragma unroll
+        for (int l = 0; l < 4; ++l) r1[l] = h[4 + l] * h[4 + l];
+#pragma unroll
+        for (int idx = 8; idx < 32; idx += 8) {
+            if (idx < aligned2) {
+#pragma unroll
+                for (int l = 0; l < 4; ++l) { r0[l] = r0[l] + h[idx + l] * h[idx + l]; r1[l] = r1[l] + h[idx + 4 + l] * h[idx + 4 + l]; }
+            }
+        }
+#pragma unroll
+        for (int l = 0; l < 4; ++l) r0[l] = r0[l] + r1[l];
+        if (aligned > aligned2) {
+#pragma unroll
+            for (int idx = 0; idx < 32; idx += 8) {
+                if (idx == aligned2) {
+#pragma unroll
+                    for (int l = 0; l < 4; ++l) r0[l] = r0[l] + h[idx + l] * h[idx + l];
+                }
+            }
+        }
+    }
+    float s = (r0[0] + r0[2]) + (r0[1] + r0[3]);
+#pragma unroll
+    for (int i = 4; i < 32; ++i) if (i >= aligned && i < nb) s = s + h[i] * h[i];
+    return s;
+}
+
+// RIFTEstimation(radius): one thread per query walks its (d2, idx)-sorted row; per neighbour the gradient magnitude and the angle
+// to (p - p0), the bilinear spread over (distance, gradient) bins in PCL's loop order; the nd x ng histogram (<= 32 floats) is kept
+// in registers -- bin indices are run-time values, so every add goes through an unrolled compare over the 32 slots -- then
+// normalised and written in PCL's order, bin = gradient_bin * nd + distance_bin (the column-major storage of Eigen's nd x ng matrix).
+__global__ void __launch_bounds__(128) rift_rows_kernel(Grid g, QueryView v, const int64_t *__restrict__ offsets, const nkey_t *__restrict__ keys,
+                                                        const uint32_t *__restrict__ inv_pos, const float4 *__restrict__ gradient, float radius,
+                                                        int nd, int ng, float *__restrict__ out) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= v.nq) return;
+    float qx, qy, qz;
+    const int64_t row = rows_query(g, v, t, qx, qy, qz);
+    const int nb = nd * ng;
+    float *o = out + row * nb;
+    const int64_t b = offsets[row], e = offsets[row + 1];
+    if (e == b) { for (int k = 0; k < nb; ++k) o[k] = CUDART_NAN_F; return; }
+    float h[32];
+#pragma unroll
+    for (int k = 0; k < 32; ++k) h[k] = 0.f;
+    const float rden = radius + 1.1920929e-07f, gden = 3.14159274f + 1.1920929e-07f;       // float(M_PI) + FLT_EPSILON
+    const float fnd = (float)nd, fng = (float)ng;
+    for (int64_t j = b; j < e; ++j) {
+        const nkey_t key = keys[j];
+        const uint32_t id = (uint32_t)key;
+        const float4 p = __ldg(g.pts + __ldg(inv_pos + id));
+        const float4 gv = __ldg(gradient + id);
+        const float mag = sqrtf(sum3(gv.x * gv.x, gv.y * gv.y, gv.z * gv.z));
+        float ux = p.x - qx, uy = p.y - qy, uz = p.z - qz;
+        const float z = sum3(ux * ux, uy * uy, uz * uz);
+        if (z > 0.f) { const float s = sqrtf(z); ux = __fdiv_rn(ux, s); uy = __fdiv_rn(uy, s); uz = __fdiv_rn(uz, s); }
+        float ang = acosf(__fdiv_rn(sum3(gv.x * ux, gv.y * uy, gv.z * uz), mag));
+        if (!isfinite(ang)) ang = 0.f;
+        const float dist = __fdiv_rn(fnd * sqrtf(__uint_as_float((uint32_t)(key >> 32))), rden);
+        const float grad = __fdiv_rn(fng * ang, gden);
+        const int dmin = max((int)ceilf(dist - 1.f), 0), dmax = min((int)floorf(dist + 1.f), nd - 1);
+        const int gmin = (int)ceilf(grad - 1.f), gmax = (int)floorf(grad + 1.f);
+        for (int gi = gmin; gi <= gmax; ++gi) {
+            const int gw = (gi + ng) % ng;
+            const float wg = 1.0f - fabsf(grad - (float)gi);
+            for (int di = dmin; di <= dmax; ++di) {
+                const float w = (1.0f - fabsf(dist - (float)di)) * wg;
+                const float add = w * mag;
+                const int bin = gw * nd + di;
+#pragma unroll
+                for (int k = 0; k < 32; ++k) if (k == bin) h[k] += add;
+            }
+        }
+    }
+    const float z = rift_sq_norm(h, nb);
+    if (z > 0.f) {
+        const float s = sqrtf(z);
+#pragma unroll
+        for (int k = 0; k < 32; ++k) h[k] = __fdiv_rn(h[k], s);
+    }
+#pragma unroll
+    for (int k = 0; k < 32; ++k) if (k < nb) o[k] = h[k];
+}
+
 // SIFT keypoint snap: lowest original index with sqrt(double(dx)^2 + double(dy)^2 + double(dz)^2) < thr
 __global__ void __launch_bounds__(128) first_within_kernel(Grid g, QueryView v, double thr, float r2_cover, int R0, int32_t *__restrict__ out) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -439,6 +593,7 @@ __global__ void ece_label_kernel(Grid g, const uint32_t *__restrict__ parent, co
     labels[__float_as_int(__ldg(g.pts + t).w)] = (int32_t)rank_of_root[parent[t]];
 }
 __global__ void fill_u32_kernel(uint32_t *p, int64_t n, uint32_t v) { int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = v; }
+__global__ void fill_f4_kernel(float4 *p, int64_t n, float4 v) { int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = v; }
 
 static int heap_threads(int k) {
     int t = (int)((96 * 1024) / ((size_t)k * sizeof(nkey_t)));
@@ -675,6 +830,91 @@ int pcc_normals_radius(pcc_index *idx, const void *q, int64_t nq, int stride_byt
     }
     timer.stop();
     if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * 16, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
+    return PCC_OK;
+}
+
+// shared front half of the two descriptor consumers: sorted radius rows of the batch in idx->keys64, offsets in idx->out_l
+static int descriptor_rows(pcc_index *idx, const Queries &qs, double radius, int64_t **d_off_out, nkey_t **keys_out, cudaStream_t s) {
+    if (!idx->inv_valid) PCC_TRY(rebuild_inverse(idx, s));
+    PCC_TRY(idx->out_l.reserve((size_t)(qs.rows + 1) * 8));
+    int64_t *d_off = idx->out_l.as<int64_t>();
+    PCC_TRY(radius_offsets(idx, qs, radius, 0, d_off, s));
+    int64_t *h = (int64_t *)idx->h_pinned;
+    PCC_CUDA(cudaMemcpyAsync(h, d_off + qs.rows, 8, cudaMemcpyDeviceToHost, s));
+    PCC_CUDA(cudaStreamSynchronize(s));
+    *d_off_out = d_off;
+    return radius_rows(idx, qs, radius, 0, 1, d_off, h[0], keys_out, s);
+}
+// host inputs of the descriptor consumers go to device scratch: stage4 is free after pcc_build, sel_params is only used inside
+// the k > 32 kNN selection (the radius rows below touch neither)
+static int stage_in(pcc::Buf &buf, const void *src, size_t bytes, int mem, cudaStream_t s, const void **dev) {
+    if (mem != PCC_HOST) { *dev = src; return PCC_OK; }
+    PCC_TRY(buf.reserve(std::max<size_t>(bytes, 16)));
+    PCC_CUDA(cudaMemcpyAsync(buf.p, src, bytes, cudaMemcpyHostToDevice, s));
+    *dev = buf.p;
+    return PCC_OK;
+}
+
+int pcc_intensity_gradient(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *intensity, const float *normals4,
+                           float *out, int mem, void *stream) {
+    PCC_TRY(check_common(idx));
+    if (!(radius >= 0)) return fail(PCC_ERR_INVALID, "bad radius");
+    cudaStream_t s = (cudaStream_t)stream;
+    Queries qs;
+    PCC_TRY(prepare_queries(idx, q, nq, stride_bytes, mem, s, &qs));
+    if (qs.rows == 0) return PCC_OK;
+    if (!out || !intensity || !normals4) return fail(PCC_ERR_INVALID, "intensity / normals / output pointer is NULL");
+    const void *d_int = nullptr, *d_nrm = nullptr;
+    PCC_TRY(stage_in(idx->stage4, intensity, (size_t)idx->n_input * 4, mem, s, &d_int));
+    PCC_TRY(stage_in(idx->sel_params, normals4, (size_t)qs.rows * 16, mem, s, &d_nrm));
+    KernelTimer timer(idx, s);
+    int64_t *d_off = nullptr; nkey_t *keys = nullptr;
+    PCC_TRY(descriptor_rows(idx, qs, radius, &d_off, &keys, s));
+    float4 *od = (float4 *)out;
+    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * 16)); od = idx->out_f.as<float4>(); }
+    if (qs.self && !idx->all_rows_indexed) {
+        fill_f4_kernel<<<nblocks(qs.rows, 256), 256, 0, s>>>(od, qs.rows, make_float4(NAN, NAN, NAN, 0.f));
+        PCC_LAUNCHED();
+    }
+    if (qs.nq > 0) {
+        gradient_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), (const float *)d_int,
+                                                                 (const float4 *)d_nrm, od);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    timer.stop();
+    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * 16, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
+    return PCC_OK;
+}
+
+int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *gradient4, int n_distance_bins, int n_gradient_bins,
+             float *out, int mem, void *stream) {
+    PCC_TRY(check_common(idx));
+    if (!(radius >= 0)) return fail(PCC_ERR_INVALID, "bad radius");
+    if (n_distance_bins < 1 || n_gradient_bins < 1 || n_distance_bins * n_gradient_bins > 32)
+        return fail(PCC_ERR_INVALID, "RIFT bins %d x %d: the histogram holds 1..32 bins (pcl::Histogram<32>)", n_distance_bins, n_gradient_bins);
+    cudaStream_t s = (cudaStream_t)stream;
+    Queries qs;
+    PCC_TRY(prepare_queries(idx, q, nq, stride_bytes, mem, s, &qs));
+    if (qs.rows == 0) return PCC_OK;
+    if (!out || !gradient4) return fail(PCC_ERR_INVALID, "gradient / output pointer is NULL");
+    const int nb = n_distance_bins * n_gradient_bins;
+    const void *d_grad = nullptr;
+    PCC_TRY(stage_in(idx->stage4, gradient4, (size_t)idx->n_input * 16, mem, s, &d_grad));
+    KernelTimer timer(idx, s);
+    int64_t *d_off = nullptr; nkey_t *keys = nullptr;
+    PCC_TRY(descriptor_rows(idx, qs, radius, &d_off, &keys, s));
+    float *od = out;
+    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * nb * 4)); od = idx->out_f.as<float>(); }
+    if (qs.self && !idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0xFF, (size_t)qs.rows * nb * 4, s));
+    if (qs.nq > 0) {
+        rift_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), (const float4 *)d_grad,
+                                                             (float)radius, n_distance_bins, n_gradient_bins, od);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    timer.stop();
+    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * nb * 4, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
     return PCC_OK;
 }
 

@@ -167,6 +167,40 @@ class GridSearch:
         check(self._L.pcc_normals_radius(self._h, ptr, nq, stride, float(radius), vp, op, mem, _stream(self.device)))
         return out
 
+    def _per_row(self, a, mem, rows: int, cols: int, dtype=np.float32):
+        """An input table of the descriptor consumers in the memory kind of the call: [rows, cols] float32, contiguous."""
+        if mem == DEVICE:
+            t = a if _is_cuda(a) else torch.as_tensor(np.asarray(a), device=f"cuda:{self.device}")
+            t = t.to(device=f"cuda:{self.device}", dtype=torch.float32).reshape(rows, -1)
+            if t.shape[1] < cols:
+                t = torch.nn.functional.pad(t, (0, cols - t.shape[1]))
+            t = t[:, :cols].contiguous()
+            return t, t.data_ptr()
+        h = a.detach().cpu().numpy() if _is_cuda(a) else np.asarray(a)
+        h = np.asarray(h, dtype).reshape(rows, -1)
+        out = np.zeros((rows, cols), dtype)
+        out[:, : min(cols, h.shape[1])] = h[:, :cols]
+        return out, out.ctypes.data
+
+    def intensityGradient(self, queries, radius: float, intensity, normals):
+        """IntensityGradientEstimation (src/comparator.cpp:649-656): intensity[n_input] per input row of the indexed cloud,
+        normals[rows, >=3] of the queries (rows = n_input for queries=None).  Returns [rows, 4] = gx, gy, gz, 0."""
+        ptr, nq, stride, mem, keep, rows = self._queries(queries)
+        it, ip = self._per_row(intensity, mem, self._n_input, 1)
+        nm, nmp = self._per_row(normals, mem, rows, 4)
+        out, op = self._alloc(mem, (rows, 4), np.float32)
+        check(self._L.pcc_intensity_gradient(self._h, ptr, nq, stride, float(radius), ip, nmp, op, mem, _stream(self.device)))
+        return out
+
+    def rift(self, queries, radius: float, gradients, nr_distance_bins: int = 4, nr_gradient_bins: int = 8):
+        """RIFTEstimation (src/comparator.cpp:659-673): gradients[n_input, >=3] per input row of the indexed cloud.  Returns
+        [rows, nd*ng] in PCL's histogram order (gradient bin outer, distance bin inner); NaN rows for queries without neighbours."""
+        ptr, nq, stride, mem, keep, rows = self._queries(queries)
+        gt, gp = self._per_row(gradients, mem, self._n_input, 4)
+        out, op = self._alloc(mem, (rows, max(int(nr_distance_bins) * int(nr_gradient_bins), 1)), np.float32)
+        check(self._L.pcc_rift(self._h, ptr, nq, stride, float(radius), gp, int(nr_distance_bins), int(nr_gradient_bins), op, mem, _stream(self.device)))
+        return out
+
     def icpStep(self, source, T_apply=None, want_correspondences: bool = False):
         """One correspondence pass against the indexed (target) cloud; `source` is moved in place by T_apply."""
         ptr, ns, stride, mem, keep = _rows(source)
@@ -344,6 +378,35 @@ def match_rift_features_knn(desc1, desc2, threshold: float = 0.05, match_dims: i
         idx, d2 = idx.cpu().numpy(), d2.cpu().numpy()
     keep = (idx >= 0) & (d2 < np.float32(threshold))
     return [0] + idx[keep].tolist()
+
+
+def rgb_to_intensity(rgb):
+    """PCL 1.7 PointXYZRGBtoXYZI (src/comparator.cpp:597): 0.299f r + 0.587f g + 0.114f b, evaluated left to right in fp32.
+    rgb[n, 3] uint8 (r, g, b) -> float32[n]."""
+    c = np.asarray(rgb.cpu().numpy() if _is_cuda(rgb) else rgb).reshape(-1, 3).astype(np.float32)
+    return ((np.float32(0.299) * c[:, 0] + np.float32(0.587) * c[:, 1]) + np.float32(0.114) * c[:, 2]).astype(np.float32)
+
+
+def process_rift(xyz, rgb, normal_radius: float = 0.03, gradient_radius: float = 0.03, rift_radius: float = 0.05, nr_distance_bins: int = 4,
+                 nr_gradient_bins: int = 8, device: int = 0, stages: dict | None = None):
+    """processRIFT (src/comparator.cpp:590-684) on the GPU: intensity (:597) -> NormalEstimation r 0.03 (:628-635) -> drop the rows
+    whose normal is NaN (:637-646) -> IntensityGradientEstimation r 0.03 (:649-656) -> RIFTEstimation r 0.05, 4 x 8 bins (:659-673)
+    -> drop the rows with a non-finite bin (:674-681).  The gradient and RIFT stages search the filtered cloud, so the index is
+    rebuilt on it.  Returns (descriptors [m, nd*ng] float32, kept_rows int64 into xyz); m is the reference's "Number of
+    descriptors".  `stages` (a dict) receives the intermediate arrays."""
+    xyz = np.ascontiguousarray(np.asarray(xyz.cpu().numpy() if _is_cuda(xyz) else xyz, np.float32)[:, :3])
+    inten = rgb_to_intensity(rgb)
+    s0 = GridSearch(device).setInputCloud(xyz, cell_hint=normal_radius)
+    normals = s0.normalsRadius(None, normal_radius)
+    keep1 = np.flatnonzero(np.isfinite(normals[:, :3]).all(1))
+    xyz1 = np.ascontiguousarray(xyz[keep1])
+    s1 = GridSearch(device).setInputCloud(xyz1, cell_hint=rift_radius)
+    grad = s1.intensityGradient(None, gradient_radius, inten[keep1], normals[keep1])
+    desc = s1.rift(None, rift_radius, grad, nr_distance_bins, nr_gradient_bins)
+    keep2 = np.flatnonzero(np.isfinite(desc).all(1))
+    if stages is not None:
+        stages.update(intensity=inten, normals=normals, kept_normals=keep1, gradients=grad, descriptors_all=desc)
+    return desc[keep2], keep1[keep2].astype(np.int64)
 
 
 def umeyama_from_sums(sums, count: int):
