@@ -22,7 +22,9 @@
 #ifndef PCC_GRID_SEARCH_HPP_
 #define PCC_GRID_SEARCH_HPP_
 
+#include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <cstdint>
 #include <limits>
 #include <memory>
@@ -538,6 +540,44 @@ class RIFTEstimation {
     const std::vector<IntensityGradient> *gradient_ = nullptr;
     double radius_ = 0;
     int nd_ = 4, ng_ = 8;
+};
+
+// pcl::PointWithScale: a SIFT keypoint (x, y, z of the octave point and the scale it was detected at)
+struct PointWithScale { float x, y, z, scale; };
+
+// pcl::SIFTKeypoint<PointT, PointWithScale>::compute as processSift configures it (src/comparator.cpp:449-465): one call
+// (pcc_sift_keypoints) runs the whole octave loop on the GPU.  The class owns its workspace index, as VoxelGrid does; after compute
+// it indexes the last octave's grid.  setSearchMethod is accepted for PCL's call pattern and not used: PCL 1.7 re-points the tree at
+// every octave's grid itself.  PointT needs PCL's packed `rgb` member.  Defaults are the reference's parameters.
+template <typename PointT>
+class SIFTKeypoint {
+  public:
+    explicit SIFTKeypoint(int device = 0) { check(pcc_create(device, &ws_)); }
+    ~SIFTKeypoint() { pcc_destroy(ws_); }
+    SIFTKeypoint(const SIFTKeypoint &) = delete;
+    SIFTKeypoint &operator=(const SIFTKeypoint &) = delete;
+    void setInputCloud(const typename search::GridSearch<PointT>::PointCloudConstPtr &cloud) { input_ = cloud; }
+    void setSearchMethod(const typename search::GridSearch<PointT>::Ptr &) {}
+    void setScales(float min_scale, int nr_octaves, int nr_scales_per_octave) { min_scale_ = min_scale; nr_octaves_ = nr_octaves; nr_scales_per_octave_ = nr_scales_per_octave; }
+    void setMinimumContrast(float min_contrast) { min_contrast_ = min_contrast; }
+    void compute(std::vector<PointWithScale> &out) {
+        if (!input_) throw Error("SIFTKeypoint: no input cloud");
+        const int64_t n = (int64_t)input_->points.size();
+        int64_t cap = std::max<int64_t>(n, 1), found = 0;
+        for (;;) {                                   // the keypoint count is known after the call: retry once with room for all
+            out.resize((size_t)cap);
+            check(pcc_sift_keypoints(ws_, input_->points.data(), n, (int)sizeof(PointT), (int)offsetof(PointT, rgb), min_scale_, nr_octaves_,
+                                     nr_scales_per_octave_, min_contrast_, reinterpret_cast<float *>(out.data()), cap, &found, PCC_HOST, nullptr));
+            if (found <= cap) break;
+            cap = found;
+        }
+        out.resize((size_t)found);
+    }
+  private:
+    pcc_index *ws_ = nullptr;
+    typename search::GridSearch<PointT>::PointCloudConstPtr input_;
+    float min_scale_ = 0.005f, min_contrast_ = 0.001f;
+    int nr_octaves_ = 5, nr_scales_per_octave_ = 5;
 };
 
 // matchRIFTFeaturesKnn (src/comparator.cpp:560-588): KdTreeFLANN<Histogram<32>> over descriptors1, nearestKSearch(k = 1) for every

@@ -110,6 +110,34 @@ int pcc_intensity_gradient(pcc_index *idx, const void *q, int64_t nq, int stride
 int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *gradient4,
              int n_distance_bins, int n_gradient_bins, float *out, int mem, void *stream);
 
+/* SIFTKeypoint<PointXYZRGB, PointWithScale> (src/comparator.cpp:449-465: min_scale 0.005, 5 octaves, 5 scales per octave,
+ * min_contrast 0.001) [up].  DESIGN.md section 2 records the reading of PCL's sift_keypoint.hpp these restate.
+ *
+ * computeScaleSpace over the indexed cloud itself: values[n_input] = one field value per INPUT row (SIFTKeypointFieldSelector);
+ * scales[n_scales] (HOST array in either memory mode, positive and ascending, 2 <= n_scales <= 16) is one octave's scale table.
+ * sigma^2 = powf(scale, 2.0f) and the cutoff 9 sigma^2 are formed on the host; each point's (d2, idx)-sorted radius row at
+ * max_radius = 3.0f * scales[n_scales-1] is walked once: scale s sums w = expf((-0.5f d2) / sigma_s^2) over the neighbours with
+ * d2 <= 9 sigma_s^2, response_s = sum(value w) / sum(w).  out[n_input * (n_scales-1)] row-major, dog[:, s-1] = response_s -
+ * response_{s-1}; rows of skipped (non-finite) inputs are NaN.  expf is the fp64-evaluated restatement of pcc_device.cuh
+ * (sift_expf), which may differ from a libm expf by one ulp. */
+int pcc_sift_dog(pcc_index *idx, const float *values, const float *scales, int n_scales, float *out, int mem, void *stream);
+/* findScaleSpaceExtrema: dog[n_input * n_cols] row-major over the indexed cloud (1 <= n_cols <= 15).  Per point the min and max of
+ * every column over its min(25, pcc_size) nearest points (pcc_knn, q == NULL; ties by (d2, index)); the point is a keypoint at
+ * column c in 1..n_cols-2 when |v| >= min_contrast and (v == min[c] && v < min[c-1] && v < min[c+1]) or else (v == max[c] &&
+ * v > max[c-1] && v > max[c+1]).  (out_row, out_col) in (row, column) order; *n_found is always the full count, at most `cap`
+ * entries are written. */
+int pcc_sift_extrema(pcc_index *idx, const float *dog, int n_cols, float min_contrast, int32_t *out_row, int32_t *out_col, int64_t cap,
+                     int64_t *n_found, int mem, void *stream);
+/* detectKeypoints: the octave loop over pts[n] (rows of stride_bytes >= 16 with x, y, z first and the packed 0x00RRGGBB colour word at
+ * rgb_offset_bytes -- pcl::PointXYZRGB: stride 32, offset 16).  scale = min_scale; per octave: VoxelGrid(leaf = scale, rgb averaged)
+ * of the previous octave's cloud (the input for the first), stop below 25 points, index the result, scales[i] = scale *
+ * powf(2.0f, (1.0f * i - 1.0f) / nr_scales_per_octave) for i < nr_scales_per_octave + 3, pcc_sift_dog on the field values
+ * float(299 r + 587 g + 114 b) / 1000.0f, pcc_sift_extrema, then scale *= 2.  out4 rows = (x, y, z, scales[column]) in (octave,
+ * point, column) order; *n_keypoints is the full count, at most `cap` rows are written.  nr_scales_per_octave <= 13.
+ * `idx` is the workspace: the call rebuilds it per octave and leaves it indexing the last octave's grid. */
+int pcc_sift_keypoints(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, int rgb_offset_bytes, float min_scale, int nr_octaves,
+                       int nr_scales_per_octave, float min_contrast, float *out4, int64_t cap, int64_t *n_keypoints, int mem, void *stream);
+
 /* CorrespondenceEstimation::determineCorrespondences + the sums TransformationEstimationSVD needs
  * (src/comparator.cpp:1091-1096) [up].  Each source point is first moved by the row-major 4x4 `T_apply`
  * (IterativeClosestPoint::transformCloud arithmetic; NULL = identity) IN PLACE when `src_inout` is device

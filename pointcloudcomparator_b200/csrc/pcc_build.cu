@@ -325,7 +325,9 @@ void pcc_destroy(pcc_index *idx) {
     if (idx->shadow) { pcc_index *sh = idx->shadow; idx->shadow = nullptr; pcc_destroy(sh); }
     for (int i = 0; i < 2; ++i) if (idx->pipe_stream[i]) cudaStreamDestroy(idx->pipe_stream[i]);
     Buf *bufs[] = {&idx->pts, &idx->cell_start, &idx->occ, &idx->occ2, &idx->cstart, &idx->raw, &idx->stage4, &idx->cellrank, &idx->qbuf, &idx->qkeys, &idx->qkeys2, &idx->qperm, &idx->qperm2,
-                   &idx->cub_tmp, &idx->out_i, &idx->out_f, &idx->out_l, &idx->keys64, &idx->keys64b, &idx->misc, &idx->parent, &idx->inv_pos, &idx->sel_params, &idx->icp_prior, &idx->calib};
+                   &idx->cub_tmp, &idx->out_i, &idx->out_f, &idx->out_l, &idx->keys64, &idx->keys64b, &idx->misc, &idx->parent, &idx->inv_pos, &idx->sel_params, &idx->icp_prior, &idx->calib,
+                   &idx->sift_cloud[0], &idx->sift_cloud[1], &idx->sift_val, &idx->sift_dog, &idx->sift_in, &idx->sift_nbr, &idx->sift_d2, &idx->sift_flag, &idx->sift_pos,
+                   &idx->sift_row, &idx->sift_col, &idx->sift_kp};
     for (Buf *b : bufs) b->release();
     if (idx->h_pinned) cudaFreeHost(idx->h_pinned);
     if (idx->aux_stream) cudaStreamDestroy(idx->aux_stream);

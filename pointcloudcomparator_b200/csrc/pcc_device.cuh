@@ -548,4 +548,29 @@ __device__ __forceinline__ void colpiv_qr_solve(float a[9], const float b[3], fl
     }
 }
 
+// expf for SIFTKeypoint's Gaussian weights, restated so that the CPU oracle (descriptor_oracle.c orc_sift_expf) computes the same
+// bits: fp64 with every operation separately rounded -- Cody-Waite reduction x = k ln2 + r (fdlibm's split of ln2), Horner Taylor
+// polynomial to r^11 on |r| <= ln2/2, exact scaling by 2^k -- then ONE rounding to fp32.  The fp64 error (~1e-15 relative) makes
+// the result the correctly rounded expf except within ~1e-15 of an fp32 rounding midpoint, so it can differ by one ulp from a
+// libm expf.  Valid for x in [-80, 80]; SIFT only calls it on [-4.6, 0].
+__device__ __forceinline__ float sift_expf(float x) {
+    const double xd = (double)x;
+    const double k = rint(__dmul_rn(xd, 1.4426950408889634));
+    const double r = __dsub_rn(__dsub_rn(xd, __dmul_rn(k, 0.6931471803691238)), __dmul_rn(k, 1.9082149292705877e-10));
+    double p = 2.505210838544172e-08;
+    p = __dadd_rn(__dmul_rn(p, r), 2.755731922398589e-07);
+    p = __dadd_rn(__dmul_rn(p, r), 2.7557319223985893e-06);
+    p = __dadd_rn(__dmul_rn(p, r), 2.48015873015873e-05);
+    p = __dadd_rn(__dmul_rn(p, r), 0.0001984126984126984);
+    p = __dadd_rn(__dmul_rn(p, r), 0.001388888888888889);
+    p = __dadd_rn(__dmul_rn(p, r), 0.008333333333333333);
+    p = __dadd_rn(__dmul_rn(p, r), 0.041666666666666664);
+    p = __dadd_rn(__dmul_rn(p, r), 0.16666666666666666);
+    p = __dadd_rn(__dmul_rn(p, r), 0.5);
+    p = __dadd_rn(__dmul_rn(p, r), 1.0);
+    p = __dadd_rn(__dmul_rn(p, r), 1.0);
+    const double two_k = __hiloint2double(((int)k + 1023) << 20, 0);
+    return __double2float_rn(__dmul_rn(p, two_k));
+}
+
 }  // namespace pcc

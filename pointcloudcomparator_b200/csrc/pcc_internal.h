@@ -69,6 +69,8 @@ struct pcc_index {
     bool occ_valid = false;
     // scratch (grow-only, reused by every call on this index; calls on one index are serialised by the caller per stream)
     pcc::Buf raw, stage4, cellrank, qbuf, qkeys, qkeys2, qperm, qperm2, cub_tmp, out_i, out_f, out_l, keys64, keys64b, misc, parent, inv_pos, sel_params, icp_prior, calib;
+    // pcc_sift_*: the octave clouds (ping-pong, float4 x, y, z, packed rgb) live outside the scratch pcc_voxel_grid and pcc_build reuse
+    pcc::Buf sift_cloud[2], sift_val, sift_dog, sift_in, sift_nbr, sift_d2, sift_flag, sift_pos, sift_row, sift_col, sift_kp;
     uint64_t grid_gen = 0;     // bumped by pcc_build / pcc_adopt
     void *comm = nullptr;      // ncclComm_t handed to pcc_comm_init (not owned); rank / world of this process in it
     int comm_rank = 0, comm_world = 1;

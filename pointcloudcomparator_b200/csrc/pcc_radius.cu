@@ -484,6 +484,47 @@ __global__ void __launch_bounds__(128) rift_rows_kernel(Grid g, QueryView v, con
     for (int k = 0; k < 32; ++k) if (k < nb) o[k] = h[k];
 }
 
+// per-scale constants of SIFTKeypoint::computeScaleSpace, computed on the host with PCL's libm calls (pcc_sift_dog)
+struct SiftScales { float sigma_sqr[16]; float cutoff[16]; };
+
+// SIFTKeypoint::computeScaleSpace: one thread per point walks its (d2, idx)-sorted row once.  PCL sums each scale over the row
+// prefix with d2 <= 9 sigma^2 (it breaks at the first neighbour beyond); the cutoffs grow with the scale, so a neighbour feeds a
+// suffix of the scales and every (num, den) pair sees the same terms in the same order as PCL's per-scale loop.
+__global__ void __launch_bounds__(128) sift_dog_rows_kernel(Grid g, QueryView v, const int64_t *__restrict__ offsets, const nkey_t *__restrict__ keys,
+                                                            const float *__restrict__ values, SiftScales sc, int ns, float *__restrict__ out) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= v.nq) return;
+    float qx, qy, qz;
+    const int64_t row = rows_query(g, v, t, qx, qy, qz);
+    const int64_t b = offsets[row], e = offsets[row + 1];
+    float num[16], den[16];
+#pragma unroll
+    for (int s = 0; s < 16; ++s) { num[s] = 0.f; den[s] = 0.f; }
+    for (int64_t j = b; j < e; ++j) {
+        const nkey_t key = keys[j];
+        const float d2 = __uint_as_float((uint32_t)(key >> 32));
+        const float val = __ldg(values + (uint32_t)key);
+#pragma unroll
+        for (int s = 0; s < 16; ++s) {
+            if (s < ns && d2 <= sc.cutoff[s]) {
+                const float w = sift_expf(__fdiv_rn(__fmul_rn(-0.5f, d2), sc.sigma_sqr[s]));
+                num[s] = __fadd_rn(num[s], __fmul_rn(val, w));
+                den[s] = __fadd_rn(den[s], w);
+            }
+        }
+    }
+    float *o = out + row * (ns - 1);
+    float prev = 0.f;
+#pragma unroll
+    for (int s = 0; s < 16; ++s) {
+        if (s < ns) {
+            const float resp = __fdiv_rn(num[s], den[s]);
+            if (s > 0) o[s - 1] = __fsub_rn(resp, prev);
+            prev = resp;
+        }
+    }
+}
+
 // SIFT keypoint snap: lowest original index with sqrt(double(dx)^2 + double(dy)^2 + double(dz)^2) < thr
 __global__ void __launch_bounds__(128) first_within_kernel(Grid g, QueryView v, double thr, float r2_cover, int R0, int32_t *__restrict__ out) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -915,6 +956,41 @@ int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double
     }
     timer.stop();
     if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * nb * 4, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
+    return PCC_OK;
+}
+
+int pcc_sift_dog(pcc_index *idx, const float *values, const float *scales, int n_scales, float *out, int mem, void *stream) {
+    PCC_TRY(check_common(idx));
+    if (!scales || n_scales < 2 || n_scales > 16) return fail(PCC_ERR_INVALID, "SIFT scale space of %d scales: 2..16 are supported", n_scales);
+    SiftScales sc{};
+    for (int i = 0; i < n_scales; ++i) {
+        if (!(scales[i] > 0.f) || !std::isfinite(scales[i]) || (i > 0 && !(scales[i] >= scales[i - 1])))
+            return fail(PCC_ERR_INVALID, "SIFT scales must be positive, finite and ascending (scale %d = %g)", i, (double)scales[i]);
+        sc.sigma_sqr[i] = powf(scales[i], 2.0f);                 // computeScaleSpace: sigma_sqr = powf (scales[i_scale], 2.0f)
+        sc.cutoff[i] = 9 * sc.sigma_sqr[i];                      // if (dist_sqr <= 9*sigma_sqr)
+    }
+    const double radius = (double)(3.0f * scales[n_scales - 1]);      // max_radius = 3.0f * scales.back (), a float handed to radiusSearch
+    cudaStream_t s = (cudaStream_t)stream;
+    Queries qs;
+    PCC_TRY(prepare_queries(idx, nullptr, 0, 16, mem, s, &qs));
+    if (qs.rows == 0) return PCC_OK;
+    if (!out || !values) return fail(PCC_ERR_INVALID, "values / output pointer is NULL");
+    const int nc = n_scales - 1;
+    const void *d_val = nullptr;
+    PCC_TRY(stage_in(idx->stage4, values, (size_t)idx->n_input * 4, mem, s, &d_val));
+    KernelTimer timer(idx, s);
+    int64_t *d_off = nullptr; nkey_t *keys = nullptr;
+    PCC_TRY(descriptor_rows(idx, qs, radius, &d_off, &keys, s));
+    float *od = out;
+    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * nc * 4)); od = idx->out_f.as<float>(); }
+    if (!idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0xFF, (size_t)qs.rows * nc * 4, s));
+    if (qs.nq > 0) {
+        sift_dog_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, (const float *)d_val, sc, n_scales, od);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    timer.stop();
+    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * nc * 4, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
     return PCC_OK;
 }
 

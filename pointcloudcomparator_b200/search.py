@@ -11,6 +11,7 @@ The C++ twin that a PCL build would actually link is include/pcc/grid_search.hpp
 from __future__ import annotations
 
 import ctypes as C
+import ctypes.util as ctypes_util
 
 import numpy as np
 
@@ -200,6 +201,30 @@ class GridSearch:
         out, op = self._alloc(mem, (rows, max(int(nr_distance_bins) * int(nr_gradient_bins), 1)), np.float32)
         check(self._L.pcc_rift(self._h, ptr, nq, stride, float(radius), gp, int(nr_distance_bins), int(nr_gradient_bins), op, mem, _stream(self.device)))
         return out
+
+    def siftDoG(self, values, scales):
+        """SIFTKeypoint::computeScaleSpace over the indexed cloud itself (src/comparator.cpp:449-465): values[n_input] (one field
+        value per input row), scales = one octave's ascending scale table (2..16 entries).  Returns [n_input, len(scales) - 1]
+        float32, dog[:, s-1] = response_s - response_{s-1}; NaN rows for skipped (non-finite) points."""
+        sc = np.ascontiguousarray(scales, np.float32).reshape(-1)
+        mem = self._mem
+        vt, vp = self._per_row(values, mem, self._n_input, 1)
+        out, op = self._alloc(mem, (self._n_input, max(sc.size - 1, 1)), np.float32)
+        check(self._L.pcc_sift_dog(self._h, vp, sc.ctypes.data, int(sc.size), op, mem, _stream(self.device)))
+        return out
+
+    def siftExtrema(self, dog, min_contrast: float = 0.001):
+        """SIFTKeypoint::findScaleSpaceExtrema over the indexed cloud: dog[n_input, n_cols] -> (rows, columns) int32 in (row,
+        column) order, the points that are DoG extrema among their 25 nearest neighbours."""
+        mem = self._mem
+        n_cols = int(dog.shape[1])
+        dt, dp = self._per_row(dog, mem, self._n_input, n_cols)
+        cap = max(self._n_input * max(n_cols - 2, 0), 1)
+        rows, rp = self._alloc(mem, (cap,), np.int32)
+        cols, cp = self._alloc(mem, (cap,), np.int32)
+        found = C.c_int64()
+        check(self._L.pcc_sift_extrema(self._h, dp, n_cols, float(min_contrast), rp, cp, cap, C.byref(found), mem, _stream(self.device)))
+        return rows[: found.value], cols[: found.value]
 
     def icpStep(self, source, T_apply=None, want_correspondences: bool = False):
         """One correspondence pass against the indexed (target) cloud; `source` is moved in place by T_apply."""
@@ -407,6 +432,84 @@ def process_rift(xyz, rgb, normal_radius: float = 0.03, gradient_radius: float =
     if stages is not None:
         stages.update(intensity=inten, normals=normals, kept_normals=keep1, gradients=grad, descriptors_all=desc)
     return desc[keep2], keep1[keep2].astype(np.int64)
+
+
+def sift_field_values(rgb):
+    """PCL 1.7 SIFTKeypointFieldSelector<PointXYZRGB>: float(299 r + 587 g + 114 b) / 1000.0f (integer sum, one fp32 division).
+    Not the XYZRGB -> XYZI weights of rgb_to_intensity.  rgb[n, 3] uint8 (r, g, b) -> float32[n]."""
+    c = np.asarray(rgb.cpu().numpy() if _is_cuda(rgb) else rgb).reshape(-1, 3).astype(np.int64)
+    return ((299 * c[:, 0] + 587 * c[:, 1] + 114 * c[:, 2]).astype(np.float32) / np.float32(1000.0)).astype(np.float32)
+
+
+_libm = None
+
+
+def sift_scales(base_scale: float, nr_scales_per_octave: int = 5):
+    """One octave's scale table as detectKeypointsForOctave builds it: base_scale * powf(2.0f, (1.0f * i - 1.0f) / nr_scales_per_octave)
+    for i < nr_scales_per_octave + 3, with the C library's powf (the one libpcc_search calls), float32."""
+    global _libm
+    if _libm is None:
+        _libm = C.CDLL(ctypes_util.find_library("m"))
+        _libm.powf.argtypes, _libm.powf.restype = [C.c_float, C.c_float], C.c_float
+    nsp = np.float32(nr_scales_per_octave)
+    e = [(np.float32(1.0) * np.float32(i) - np.float32(1.0)) / nsp for i in range(int(nr_scales_per_octave) + 3)]
+    return np.array([np.float32(base_scale) * np.float32(_libm.powf(2.0, float(x))) for x in e], np.float32)
+
+
+def _sift_rows(xyz, rgb):
+    """[n, 4] float32 (x, y, z, packed 0x00RRGGBB word): the layout pcc_sift_keypoints and every octave cloud use."""
+    xyz = np.asarray(xyz.cpu().numpy() if _is_cuda(xyz) else xyz, np.float32)
+    c = np.asarray(rgb.cpu().numpy() if _is_cuda(rgb) else rgb).reshape(-1, 3).astype(np.uint32)
+    rows = np.empty((xyz.shape[0], 4), np.float32)
+    rows[:, :3] = xyz[:, :3]
+    rows[:, 3] = ((c[:, 0] << 16) | (c[:, 1] << 8) | c[:, 2]).view(np.float32)
+    return rows
+
+
+def sift_keypoints(xyz, rgb, min_scale: float = 0.005, nr_octaves: int = 5, nr_scales_per_octave: int = 5, min_contrast: float = 0.001,
+                   device: int = 0, stages: dict | None = None):
+    """SIFTKeypoint<PointXYZRGB, PointWithScale>::compute as processSift configures it (src/comparator.cpp:449-465), one
+    pcc_sift_keypoints call: returns float32 [m, 4] = (x, y, z, scale) in (octave, point, column) order.  `stages` (a dict)
+    receives stages["octaves"], one dict per octave (cloud, scales, dog, rows, cols, keypoints), recomputed through the public
+    pieces (voxel_grid, GridSearch.siftDoG / siftExtrema); their keypoints concatenate to the returned array."""
+    rows = _sift_rows(xyz, rgb)
+    ws = GridSearch(device)
+    cap = max(rows.shape[0], 1)
+    while True:
+        out = np.empty((cap, 4), np.float32)
+        found = C.c_int64()
+        check(ws._L.pcc_sift_keypoints(ws._h, rows.ctypes.data, rows.shape[0], 16, 12, float(min_scale), int(nr_octaves), int(nr_scales_per_octave),
+                                       float(min_contrast), out.ctypes.data, cap, C.byref(found), HOST, _stream(ws.device)))
+        if found.value <= cap:
+            break
+        cap = found.value
+    if stages is not None:
+        cloud, scale, octs = rows, np.float32(min_scale), []
+        for _ in range(int(nr_octaves)):
+            cloud = voxel_grid(cloud, scale, rgb_offset_bytes=12, workspace=ws)
+            if cloud.shape[0] < 25:
+                break
+            scales = sift_scales(scale, nr_scales_per_octave)
+            s = GridSearch(device).setInputCloud(cloud, cell_hint=float(np.float32(3) * scales[-1]))
+            dog = s.siftDoG(sift_field_values(np.stack([(cloud[:, 3].view(np.uint32) >> sh) & 255 for sh in (16, 8, 0)], 1)), scales)
+            r, c = s.siftExtrema(dog, min_contrast)
+            kp = np.column_stack([cloud[r, :3], scales[c]]).astype(np.float32)
+            octs.append(dict(cloud=cloud, scales=scales, dog=dog, rows=r, cols=c, keypoints=kp))
+            scale = np.float32(scale * np.float32(2))
+        stages["octaves"] = octs
+    return out[: found.value]
+
+
+def process_sift(xyz, rgb, snap_threshold: float = 0.05, device: int = 0, **sift_kw):
+    """processSift + the snap of processRIFTwithSIFT (src/comparator.cpp:435-469, 696-713): SIFT keypoints of the cluster, then for
+    every keypoint the first cloud point (lowest index) within 0.05 of it, -1 if none.  Returns (keypoints [m, 4], snap int32[m]):
+    what processRIFTwithSIFT holds before its descriptor chain."""
+    kp = sift_keypoints(xyz, rgb, device=device, **sift_kw)
+    if kp.shape[0] == 0:
+        return kp, np.empty(0, np.int32)
+    xyz = np.ascontiguousarray(np.asarray(xyz.cpu().numpy() if _is_cuda(xyz) else xyz, np.float32)[:, :3])
+    s = GridSearch(device).setInputCloud(xyz, cell_hint=snap_threshold)
+    return kp, s.firstWithin(np.ascontiguousarray(kp[:, :3]), snap_threshold)
 
 
 def umeyama_from_sums(sums, count: int):
