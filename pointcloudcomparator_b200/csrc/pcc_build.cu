@@ -136,7 +136,8 @@ __global__ void compact_table_kernel(const uint32_t *__restrict__ occ, const uin
     while (bits) { const int b = __ffs(bits) - 1; bits &= bits - 1; cstart[r++] = cell_start[w * 32 + b]; }
     if (w == words - 1) cstart[r] = cell_start[n_cells];
 }
-int rebuild_occupancy(pcc_index *idx, cudaStream_t s) {
+// occ bitmap from cell_start (after pcc_build / pcc_adopt)
+static int rebuild_occupancy(pcc_index *idx, cudaStream_t s) {
     const int64_t n_cells = std::max<int64_t>(idx->gh.n_cells, 1);
     const int64_t words = (n_cells + 31) / 32 + 1;
     PCC_TRY(idx->occ.reserve((size_t)words * 4));
@@ -163,6 +164,13 @@ int rebuild_occupancy(pcc_index *idx, cudaStream_t s) {
     idx->occ_valid = true;
     return PCC_OK;
 }
+int check_index(pcc_index *idx, void *stream) {
+    if (!idx) return fail(PCC_ERR_INVALID, "idx is NULL");
+    if (!idx->built) return fail(PCC_ERR_STATE, "index not built (call pcc_build first)");
+    PCC_CUDA(cudaSetDevice(idx->device));
+    if (!idx->occ_valid) PCC_TRY(rebuild_occupancy(idx, (cudaStream_t)stream));     // first query after pcc_adopt
+    return PCC_OK;
+}
 int rebuild_inverse(pcc_index *idx, cudaStream_t s) {
     PCC_TRY(idx->inv_pos.reserve((size_t)std::max<int64_t>(idx->n_input, 1) * 4));
     PCC_CUDA(cudaMemsetAsync(idx->inv_pos.p, 0xFF, (size_t)std::max<int64_t>(idx->n_input, 1) * 4, s));
@@ -185,8 +193,6 @@ __global__ void qprep_kernel(const uint8_t *__restrict__ raw, int stride, int64_
     qbuf[i] = make_float4(x, y, z, 0.f);
     if (keys) { keys[i] = finite3(x, y, z) ? cell_of(b, x, y, z) : bad_key; perm[i] = (uint32_t)i; }
 }
-
-static inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
 
 // Target points per NON-EMPTY cell.  PCC_OCC overrides it (measurement knob).
 // Surface-like clouds, measured on B200 (10 M queries on a 10 M-point surface cloud, kNN ms at target 4 / 6 / 8 / 10 / 12): k = 4: 3.46 / 2.60 /
@@ -245,7 +251,7 @@ int prepare_queries(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
     PCC_TRY(idx->qbuf.reserve((size_t)nq * sizeof(float4)));
     if (idx->reuse_order_n == nq && nq > 2048) {          // same rows as the previous pass, slightly moved: keep its order
         BinParams b0{idx->gh.ox, idx->gh.oy, idx->gh.oz, idx->gh.inv_cell, idx->gh.nx, idx->gh.ny, idx->gh.nz};
-        qprep_kernel<<<blocks_for(nq, 256), 256, 0, s>>>(raw, stride_bytes, nq, b0, (uint32_t)idx->gh.n_cells, idx->qbuf.as<float4>(), nullptr, nullptr);
+        qprep_kernel<<<nblocks(nq, 256), 256, 0, s>>>(raw, stride_bytes, nq, b0, (uint32_t)idx->gh.n_cells, idx->qbuf.as<float4>(), nullptr, nullptr);
         PCC_LAUNCHED();
         PCC_CUDA(cudaGetLastError());
         out->q = idx->qbuf.as<float4>();
@@ -258,7 +264,7 @@ int prepare_queries(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
         PCC_TRY(idx->qkeys.reserve((size_t)nq * 4)); PCC_TRY(idx->qkeys2.reserve((size_t)nq * 4));
         PCC_TRY(idx->qperm.reserve((size_t)nq * 4)); PCC_TRY(idx->qperm2.reserve((size_t)nq * 4));
     }
-    qprep_kernel<<<blocks_for(nq, 256), 256, 0, s>>>(raw, stride_bytes, nq, b, (uint32_t)idx->gh.n_cells, idx->qbuf.as<float4>(),
+    qprep_kernel<<<nblocks(nq, 256), 256, 0, s>>>(raw, stride_bytes, nq, b, (uint32_t)idx->gh.n_cells, idx->qbuf.as<float4>(),
                                                      sort ? idx->qkeys.as<uint32_t>() : nullptr, sort ? idx->qperm.as<uint32_t>() : nullptr);
     PCC_LAUNCHED();
     PCC_CUDA(cudaGetLastError());
@@ -391,7 +397,7 @@ int pcc_build(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, cons
         PCC_CUDA(cudaStreamSynchronize(s));    // h is reused below
     }
     if (m > 0) {
-        extract_kernel<<<blocks_for(m, 256), 256, 0, s>>>(raw, stride_bytes, d_indices, m, n, idx->stage4.as<float4>(), d_scal, (unsigned long long *)(d_scal + 8));
+        extract_kernel<<<nblocks(m, 256), 256, 0, s>>>(raw, stride_bytes, d_indices, m, n, idx->stage4.as<float4>(), d_scal, (unsigned long long *)(d_scal + 8));
         PCC_LAUNCHED();
         PCC_CUDA(cudaGetLastError());
     }
@@ -440,14 +446,14 @@ int pcc_build(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, cons
         PCC_TRY(idx->cell_start.reserve((size_t)(n_cells + 1) * sizeof(uint32_t)));
         PCC_CUDA(cudaMemsetAsync(idx->cell_start.p, 0, (size_t)(n_cells + 1) * sizeof(uint32_t), s));
         PCC_CUDA(cudaMemsetAsync(d_scal + 10, 0, 24, s));
-        bin_kernel<<<blocks_for(m, 256), 256, 0, s>>>(idx->stage4.as<float4>(), m, b, idx->cell_start.as<uint32_t>(), idx->cellrank.as<uint2>());
+        bin_kernel<<<nblocks(m, 256), 256, 0, s>>>(idx->stage4.as<float4>(), m, b, idx->cell_start.as<uint32_t>(), idx->cellrank.as<uint2>());
         PCC_LAUNCHED();
-        nonzero_kernel<<<(unsigned)std::min<int64_t>(blocks_for(n_cells, 256), 148 * 16), 256, 0, s>>>(idx->cell_start.as<uint32_t>(), n_cells, (unsigned long long *)(d_scal + 10));
+        nonzero_kernel<<<(unsigned)std::min<int64_t>(nblocks(n_cells, 256), 148 * 16), 256, 0, s>>>(idx->cell_start.as<uint32_t>(), n_cells, (unsigned long long *)(d_scal + 10));
         PCC_LAUNCHED();
         const bool probe_fill = autotune && !target_fixed && it == 0;     // surface or volume?  decided once, on the first grid
         if (probe_fill) {
             const int64_t stride = std::max<int64_t>(1, m / kFillSamples);
-            blockfill_kernel<<<blocks_for((m + stride - 1) / stride, 256), 256, 0, s>>>(idx->stage4.as<float4>(), m, stride, b, idx->cell_start.as<uint32_t>(), (unsigned long long *)(d_scal + 12));
+            blockfill_kernel<<<nblocks((m + stride - 1) / stride, 256), 256, 0, s>>>(idx->stage4.as<float4>(), m, stride, b, idx->cell_start.as<uint32_t>(), (unsigned long long *)(d_scal + 12));
             PCC_LAUNCHED();
         }
         PCC_CUDA(cudaGetLastError());
@@ -487,7 +493,7 @@ int pcc_build(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, cons
     PCC_CUDA(cub::DeviceScan::ExclusiveSum(idx->cub_tmp.p, tmp, idx->cell_start.as<uint32_t>(), idx->cell_start.as<uint32_t>(), (int)(n_cells + 1), s));
     g_launches += 2;
     PCC_TRY(idx->pts.reserve((size_t)nfin * sizeof(float4)));
-    scatter_kernel<<<blocks_for(m, 256), 256, 0, s>>>(idx->stage4.as<float4>(), idx->cellrank.as<uint2>(), m, idx->cell_start.as<uint32_t>(), idx->pts.as<float4>());
+    scatter_kernel<<<nblocks(m, 256), 256, 0, s>>>(idx->stage4.as<float4>(), idx->cellrank.as<uint2>(), m, idx->cell_start.as<uint32_t>(), idx->pts.as<float4>());
     PCC_LAUNCHED();
     PCC_CUDA(cudaGetLastError());
     PCC_TRY(rebuild_occupancy(idx, s));

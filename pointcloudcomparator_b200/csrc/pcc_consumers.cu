@@ -12,8 +12,6 @@
 
 namespace pcc {
 
-static inline unsigned nblocks(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
-
 // per-block (sum d, sum d*d) with the product rounded in fp32 first, as PCL's "sq_sum += distances[i] * distances[i]" does
 __global__ void sor_sums_kernel(const float *__restrict__ d, int64_t n, double *__restrict__ partials) {
     __shared__ double r0[256], r1[256];
@@ -134,12 +132,8 @@ int pcc_sor_threshold(pcc_index *idx, const float *distances, int64_t n, int64_t
     if (kept) *kept = 0;
     stats[0] = stats[1] = stats[2] = 0;
     if (n == 0) return PCC_OK;
-    const float *d = distances;
-    if (mem == PCC_HOST) {
-        PCC_TRY(idx->out_f.reserve((size_t)n * 4));
-        PCC_CUDA(cudaMemcpyAsync(idx->out_f.p, distances, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-        d = idx->out_f.as<float>();
-    }
+    const float *d = nullptr;
+    PCC_TRY(stage_in(idx->out_f, distances, (size_t)n * 4, mem, s, &d));
     const int nb = (int)std::min<int64_t>(nblocks(n, 256), 1024);
     PCC_TRY(idx->keys64b.reserve((size_t)(2 * nb + 4) * sizeof(double)));
     double *partials = idx->keys64b.as<double>(), *d_out = partials + 2 * nb;
@@ -364,22 +358,16 @@ int pcc_region_growing_rgb(const int32_t *neighbours, const float *sqr_distances
 // max_iter iterations, transformation_epsilon 0 (rotation threshold 1.0, translation threshold 0), absolute MSE
 // threshold 1e-12, relative MSE threshold -DBL_MAX (never), no rejectors, no correspondence distance limit.
 int pcc_icp_align(pcc_index *idx, const void *src, int64_t ns, int stride_bytes, int max_iter, float T16[16], int *converged, double *fitness, int *iterations, int mem, void *stream) {
-    if (!idx) return fail(PCC_ERR_INVALID, "idx is NULL");
-    if (!idx->built) return fail(PCC_ERR_STATE, "index not built (call pcc_build first)");
+    PCC_TRY(check_index(idx, stream));
     if (ns < 0 || (ns > 0 && !src) || stride_bytes < 12 || (stride_bytes & 3) || !T16) return fail(PCC_ERR_INVALID, "bad source cloud");
-    PCC_CUDA(cudaSetDevice(idx->device));
     cudaStream_t s = (cudaStream_t)stream;
     float Tfinal[16], Tstep[16];
     for (int i = 0; i < 16; ++i) Tfinal[i] = (i % 5 == 0) ? 1.f : 0.f;
     int it = 0, conv = 0;
     double fit = DBL_MAX;
     // device working copy of the source (float4 rows), moved in place every iteration like PCL's input_transformed
-    const uint8_t *raw = (const uint8_t *)src;
-    if (mem == PCC_HOST && ns > 0) {
-        PCC_TRY(idx->stage4.reserve((size_t)ns * stride_bytes));     // stage4 is free after pcc_build
-        PCC_CUDA(cudaMemcpyAsync(idx->stage4.p, src, (size_t)ns * stride_bytes, cudaMemcpyHostToDevice, s));
-        raw = idx->stage4.as<uint8_t>();
-    }
+    const uint8_t *raw = nullptr;
+    PCC_TRY(stage_in(idx->stage4, (const uint8_t *)src, (size_t)ns * stride_bytes, mem, s, &raw));     // stage4 is free after pcc_build
     PCC_TRY(idx->parent.reserve((size_t)std::max<int64_t>(ns, 1) * sizeof(float4) + 64));
     float4 *cur = idx->parent.as<float4>();
     float *d_T = (float *)(cur + std::max<int64_t>(ns, 1));

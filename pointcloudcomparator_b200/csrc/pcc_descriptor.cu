@@ -70,15 +70,13 @@ extern "C" int pcc_descriptor_nn(pcc_index *ws, const float *ref, int64_t n_ref,
     PCC_CUDA(cudaSetDevice(ws->device));
     cudaStream_t s = (cudaStream_t)stream;
     if (n_qry == 0) return PCC_OK;
-    const float *d_ref = ref, *d_qry = qry;
+    const float *d_ref = nullptr, *d_qry = nullptr;
+    PCC_TRY(stage_in(ws->raw, ref, (size_t)n_ref * stride_floats * 4, mem, s, &d_ref));
+    PCC_TRY(stage_in(ws->stage4, qry, (size_t)n_qry * stride_floats * 4, mem, s, &d_qry));
     int32_t *d_oi = out_idx; float *d_od = out_d2;
     if (mem == PCC_HOST) {
-        const size_t rb = (size_t)std::max<int64_t>(n_ref, 1) * stride_floats * 4, qb = (size_t)n_qry * stride_floats * 4;
-        PCC_TRY(ws->raw.reserve(rb)); PCC_TRY(ws->stage4.reserve(qb));
         PCC_TRY(ws->out_i.reserve((size_t)n_qry * 4)); PCC_TRY(ws->out_f.reserve((size_t)n_qry * 4));
-        if (n_ref > 0) PCC_CUDA(cudaMemcpyAsync(ws->raw.p, ref, (size_t)n_ref * stride_floats * 4, cudaMemcpyHostToDevice, s));
-        PCC_CUDA(cudaMemcpyAsync(ws->stage4.p, qry, qb, cudaMemcpyHostToDevice, s));
-        d_ref = ws->raw.as<float>(); d_qry = ws->stage4.as<float>(); d_oi = ws->out_i.as<int32_t>(); d_od = ws->out_f.as<float>();
+        d_oi = ws->out_i.as<int32_t>(); d_od = ws->out_f.as<float>();
     }
     const unsigned nb = (unsigned)((n_qry + kDescThreads - 1) / kDescThreads);
     if (dim == 3) descriptor_nn_kernel<3><<<nb, kDescThreads, 0, s>>>(d_ref, n_ref, stride_floats, d_qry, n_qry, stride_floats, d_oi, d_od);

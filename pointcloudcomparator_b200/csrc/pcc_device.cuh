@@ -49,6 +49,14 @@ __device__ __forceinline__ float grid_u(float x, float o, float inv) { return __
 __device__ __forceinline__ int grid_c(float u, int n) { return (int)fminf(fmaxf(floorf(u), 0.f), (float)(n - 1)); }
 __device__ __forceinline__ bool finite3(float x, float y, float z) { return isfinite(x) && isfinite(y) && isfinite(z); }
 
+// a prepared query batch as the kernels see it (pcc_internal.h Queries)
+struct QueryView { const float4 *q; const uint32_t *order; int64_t nq; bool self; };
+// thread t (< v.nq) -> query coordinates; returns the output row.  Self mode: sorted point t, row = its original index.
+__device__ __forceinline__ int64_t rows_query(const Grid &g, const QueryView &v, int64_t t, float &x, float &y, float &z) {
+    if (v.self) { float4 p = __ldg(g.pts + t); x = p.x; y = p.y; z = p.z; return __float_as_int(p.w); }
+    uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t; float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; return qi;
+}
+
 struct QueryCell {
     float ux, uy, uz;
     int cx, cy, cz;

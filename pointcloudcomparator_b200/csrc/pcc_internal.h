@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <algorithm>
 #include <atomic>
 #include <string>
 
@@ -118,10 +119,47 @@ struct Queries {
     bool self = false;             // queries are the indexed cloud itself: thread t handles sorted point t, row = original index
     int64_t rows = 0;              // number of output rows (nq, or n_input in self mode)
 };
-int prepare_queries(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int mem, cudaStream_t s, Queries *out);
+static inline QueryView view_of(const Queries &q) { return QueryView{q.q, q.order, q.nq, q.self}; }
+static inline unsigned nblocks(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
+// block size of the kernels that keep k keys per thread in dynamic shared memory (up to 96 KB of keys a block)
+static inline int heap_threads(int k) {
+    int t = (int)((96 * 1024) / ((size_t)k * sizeof(nkey_t)));
+    t = std::min(128, (t / 32) * 32);
+    return std::max(32, t);
+}
+template <class Kern>
+static int set_heap_smem(Kern kern) {
+    PCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));   // per device: set on every launch (cheap)
+    return PCC_OK;
+}
+// an entry's input array on the device: the caller's pointer (PCC_DEVICE), or a copy in `buf` (PCC_HOST)
+template <class T>
+static int stage_in(Buf &buf, const T *src, size_t bytes, int mem, cudaStream_t s, const T **dev) {
+    *dev = src;
+    if (mem != PCC_HOST) return PCC_OK;
+    PCC_TRY(buf.reserve(std::max<size_t>(bytes, 16)));
+    if (bytes) PCC_CUDA(cudaMemcpyAsync(buf.p, src, bytes, cudaMemcpyHostToDevice, s));
+    *dev = buf.as<T>();
+    return PCC_OK;
+}
+// per-row results are written to the caller's pointer (PCC_DEVICE) or to out_f (PCC_HOST); deliver_rows copies the
+// latter back and returns with them on the host
+template <class T>
+static int output_rows(pcc_index *idx, T *out, size_t bytes, int mem, T **dev) {
+    *dev = out;
+    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve(bytes)); *dev = idx->out_f.as<T>(); }
+    return PCC_OK;
+}
 int copy_out(void *dst, const void *src_dev, size_t bytes, int mem, cudaStream_t s);
+static inline int deliver_rows(void *out, const void *dev, size_t bytes, int mem, cudaStream_t s) {
+    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, dev, bytes, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
+    return PCC_OK;
+}
+// every entry that searches the grid: idx is a built index, its device is current, and after pcc_adopt the occupancy bitmap is
+// derived on the caller's stream (ordered after the caller's fill of cell_start, before its next kernel)
+int check_index(pcc_index *idx, void *stream);
+int prepare_queries(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int mem, cudaStream_t s, Queries *out);
 int rebuild_inverse(pcc_index *idx, cudaStream_t s);
-int rebuild_occupancy(pcc_index *idx, cudaStream_t s);   // occ bitmap from cell_start (after pcc_build / pcc_adopt)
 int comm_allreduce_f64(pcc_index *idx, double *d_buf, int n, cudaStream_t s);   // pcc_comm.cu; no-op without a communicator
 // k > 32: neighbours by selection (pcc_radius.cu); rows are sorted by (d2, index), oi / od are device pointers
 int knn_select(pcc_index *idx, const Queries &qs, int k, int32_t *oi, float *od, cudaStream_t s);

@@ -20,21 +20,18 @@
 
 namespace pcc {
 
-struct QueryView {
-    const float4 *q; const uint32_t *order; int64_t nq; bool self;
-};
-// thread t -> (query coordinates, output row); returns false for tail threads and non-finite queries
+// rows_query for the kNN kernels: false for tail threads and non-finite queries; write_empty = the row still gets (-1, +inf).
+// rows_query is called on each side of the v.self test, as in pcc_radius.cu's load_query.
 __device__ __forceinline__ bool load_query(const Grid &g, const QueryView &v, int64_t t, float &x, float &y, float &z, int64_t &row, bool &write_empty) {
     write_empty = false;
     if (t >= v.nq) return false;
-    if (v.self) { float4 p = __ldg(g.pts + t); x = p.x; y = p.y; z = p.z; row = __float_as_int(p.w); return true; }
-    uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t;
-    float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; row = qi;
+    if (v.self) { row = rows_query(g, v, t, x, y, z); return true; }
+    row = rows_query(g, v, t, x, y, z);
 #ifdef PCC_EXP_SEQROWS        // measurement build only (results land in processing order): what do the scattered 128-byte row writes cost?
     row = t;
 #endif
 #ifdef PCC_EXP_SEQQ           // measurement build only: queries read in processing order instead of gathered through `order`
-    p = __ldg(v.q + t); x = p.x; y = p.y; z = p.z;
+    { float4 p = __ldg(v.q + t); x = p.x; y = p.y; z = p.z; }
 #endif
     if (!finite3(x, y, z) || g.n == 0) { write_empty = true; return false; }
     return true;
@@ -845,18 +842,6 @@ __global__ void icp_store_kernel(const float4 *__restrict__ srcw, int64_t ns, ui
 }
 
 __global__ void fill_f32_kernel(float *p, int64_t n, float v) { int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = v; }
-static inline unsigned nblocks(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
-static inline QueryView view_of(const Queries &q) { return QueryView{q.q, q.order, q.nq, q.self}; }
-static int heap_threads(int k) {
-    int t = (int)((96 * 1024) / ((size_t)k * sizeof(nkey_t)));
-    t = std::min(128, (t / 32) * 32);
-    return std::max(32, t);
-}
-template <class Kern>
-static int set_heap_smem(Kern kern) {
-    PCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));   // per device: set on every launch (cheap)
-    return PCC_OK;
-}
 
 template <int K>
 static void launch_knn_reg(const Grid &g, const QueryView &v, int k, int32_t *oi, float *od, int vec4, cudaStream_t s) {
@@ -983,18 +968,6 @@ static int launch_knn_fast(pcc_index *idx, const Grid &g, const QueryView &v, in
 
 using namespace pcc;
 
-static int check_common(pcc_index *idx, void *stream) {
-    if (!idx) return fail(PCC_ERR_INVALID, "idx is NULL");
-    if (!idx->built) return fail(PCC_ERR_STATE, "index not built (call pcc_build first)");
-    PCC_CUDA(cudaSetDevice(idx->device));
-    if (!idx->occ_valid) PCC_TRY(rebuild_occupancy(idx, (cudaStream_t)stream));     // first query after pcc_adopt
-    return PCC_OK;
-}
-
-extern "C" {
-
-}  // extern "C"
-
 // one batch on one stream; `sync` = wait for the host copies before returning (PCC_HOST only)
 static int knn_impl(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int k, int32_t *out_idx, float *out_d2, int *k_eff, int mem, cudaStream_t s, bool sync) {
     Queries qs;
@@ -1077,7 +1050,7 @@ static int knn_impl(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
 extern "C" {
 
 int pcc_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int k, int32_t *out_idx, float *out_d2, int *k_eff, int mem, void *stream) {
-    PCC_TRY(check_common(idx, stream));
+    PCC_TRY(check_index(idx, stream));
     if (k < 1 || k > PCC_MAX_K) return fail(PCC_ERR_INVALID, "k=%d outside 1..%d", k, PCC_MAX_K);
     cudaStream_t s = (cudaStream_t)stream;
     // Large host batches: two-slot pipeline, 1 Mi queries per chunk (16 MB in, k x 8 MB out), so the device->host copy of
@@ -1109,15 +1082,15 @@ int pcc_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int k, 
 }
 
 int pcc_knn_mean_dist(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int mean_k, float *out_mean, int mem, void *stream) {
-    PCC_TRY(check_common(idx, stream));
+    PCC_TRY(check_index(idx, stream));
     if (mean_k < 1 || mean_k + 1 > PCC_MAX_K) return fail(PCC_ERR_INVALID, "mean_k=%d outside 1..%d", mean_k, PCC_MAX_K - 1);
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
     PCC_TRY(prepare_queries(idx, q, nq, stride_bytes, mem, s, &qs));
     if (qs.rows == 0) return PCC_OK;
     if (!out_mean) return fail(PCC_ERR_INVALID, "output pointer is NULL");
-    float *od = out_mean;
-    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * 4)); od = idx->out_f.as<float>(); }
+    float *od = nullptr;
+    PCC_TRY(output_rows(idx, out_mean, (size_t)qs.rows * 4, mem, &od));
     if (qs.self && !idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0, (size_t)qs.rows * 4, s));
     const Grid g = idx->grid();
     const QueryView v = view_of(qs);
@@ -1144,12 +1117,11 @@ int pcc_knn_mean_dist(pcc_index *idx, const void *q, int64_t nq, int stride_byte
         PCC_CUDA(cudaGetLastError());
     }
     timer.stop();
-    if (mem == PCC_HOST) { PCC_TRY(copy_out(out_mean, od, (size_t)qs.rows * 4, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
-    return PCC_OK;
+    return deliver_rows(out_mean, od, (size_t)qs.rows * 4, mem, s);
 }
 
 int pcc_normals_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int k, const float viewpoint[3], float *out, int mem, void *stream) {
-    PCC_TRY(check_common(idx, stream));
+    PCC_TRY(check_index(idx, stream));
     if (k < 1 || k > PCC_MAX_K) return fail(PCC_ERR_INVALID, "k=%d outside 1..%d", k, PCC_MAX_K);
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
@@ -1157,8 +1129,8 @@ int pcc_normals_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
     if (qs.rows == 0) return PCC_OK;
     if (!out) return fail(PCC_ERR_INVALID, "output pointer is NULL");
     if (!idx->inv_valid) PCC_TRY(rebuild_inverse(idx, s));
-    float4 *od = (float4 *)out;
-    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * 16)); od = idx->out_f.as<float4>(); }
+    float4 *od = nullptr;
+    PCC_TRY(output_rows(idx, (float4 *)out, (size_t)qs.rows * 16, mem, &od));
     if (qs.self && !idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0xFF, (size_t)qs.rows * 16, s));   // 0xFFFFFFFF = NaN
     const float vx = viewpoint ? viewpoint[0] : 0.f, vy = viewpoint ? viewpoint[1] : 0.f, vz = viewpoint ? viewpoint[2] : 0.f;
     const Grid g = idx->grid();
@@ -1179,14 +1151,13 @@ int pcc_normals_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
         PCC_CUDA(cudaGetLastError());
     }
     timer.stop();
-    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * 16, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
-    return PCC_OK;
+    return deliver_rows(out, od, (size_t)qs.rows * 16, mem, s);
 }
 
 // src working copy lives in idx->stage4-independent buffer `parent` is reserved for clustering; ICP uses qbuf-sized `keys64b`
 int pcc_icp_step(pcc_index *idx, void *src_inout, int64_t ns, int stride_bytes, const float *T_apply, double sums[16], int64_t *count,
                  int32_t *corr_idx, float *corr_d2, int mem, void *stream) {
-    PCC_TRY(check_common(idx, stream));
+    PCC_TRY(check_index(idx, stream));
     if (ns < 0 || stride_bytes < 12 || (stride_bytes & 3)) return fail(PCC_ERR_INVALID, "bad source cloud (ns=%lld stride=%d)", (long long)ns, stride_bytes);
     if (!sums || !count) return fail(PCC_ERR_INVALID, "sums / count are NULL");
     cudaStream_t s = (cudaStream_t)stream;

@@ -11,15 +11,13 @@
 
 namespace pcc {
 
-struct QueryView { const float4 *q; const uint32_t *order; int64_t nq; bool self; };
-static inline QueryView view_of(const Queries &q) { return QueryView{q.q, q.order, q.nq, q.self}; }
-static inline unsigned nblocks(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
-
+// rows_query for the searching kernels: false for tail threads and for external queries that are not finite or meet an empty index.
+// rows_query is called on each side of the v.self test so that each inlined copy folds to one branch (a single call that branches
+// again on v.self compiles to a different block layout).
 __device__ __forceinline__ bool load_query(const Grid &g, const QueryView &v, int64_t t, float &x, float &y, float &z, int64_t &row) {
     if (t >= v.nq) return false;
-    if (v.self) { float4 p = __ldg(g.pts + t); x = p.x; y = p.y; z = p.z; row = __float_as_int(p.w); return true; }
-    uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t;
-    float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; row = qi;
+    if (v.self) { row = rows_query(g, v, t, x, y, z); return true; }
+    row = rows_query(g, v, t, x, y, z);
     return finite3(x, y, z) && g.n > 0;
 }
 
@@ -321,18 +319,12 @@ __global__ void __launch_bounds__(128) normals_rows_kernel(Grid g, QueryView v, 
                                                            const uint32_t *__restrict__ inv_pos, float vx, float vy, float vz, float4 *__restrict__ out) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= v.nq) return;
-    float x, y, z; int64_t row;
-    if (v.self) { float4 p = __ldg(g.pts + t); x = p.x; y = p.y; z = p.z; row = __float_as_int(p.w); }
-    else { uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t; float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; row = qi; }
+    float x, y, z;
+    const int64_t row = rows_query(g, v, t, x, y, z);
     const int64_t b = offsets[row], e = offsets[row + 1];
     float a[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     for (int64_t j = b; j < e; ++j) { float4 p = __ldg(g.pts + __ldg(inv_pos + (uint32_t)keys[j])); accu_add(a, p.x, p.y, p.z); }
     out[row] = normal_from_accu(a, (int)min((int64_t)INT_MAX, e - b), x, y, z, vx, vy, vz);
-}
-
-__device__ __forceinline__ int64_t rows_query(const Grid &g, const QueryView &v, int64_t t, float &x, float &y, float &z) {
-    if (v.self) { float4 p = __ldg(g.pts + t); x = p.x; y = p.y; z = p.z; return __float_as_int(p.w); }
-    uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t; float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; return qi;
 }
 
 // IntensityGradientEstimation(radius), is_dense branch: centroid and mean intensity over the sorted row, then
@@ -636,11 +628,6 @@ __global__ void ece_label_kernel(Grid g, const uint32_t *__restrict__ parent, co
 __global__ void fill_u32_kernel(uint32_t *p, int64_t n, uint32_t v) { int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = v; }
 __global__ void fill_f4_kernel(float4 *p, int64_t n, float4 v) { int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = v; }
 
-static int heap_threads(int k) {
-    int t = (int)((96 * 1024) / ((size_t)k * sizeof(nkey_t)));
-    t = std::min(128, (t / 32) * 32);
-    return std::max(32, t);
-}
 static inline int ring0(const pcc_index *idx, double radius) { return std::max(1, (int)std::ceil(radius / (double)idx->gh.cell)); }
 
 // shared by pcc_radius_count and the internal consumers: counts (device, zeroed, rows+1) -> inclusive CSR offsets
@@ -702,7 +689,7 @@ static int radius_rows(pcc_index *idx, const Queries &qs, double radius, unsigne
     if (capped) {
         if (max_nn > PCC_MAX_K) return fail(PCC_ERR_INVALID, "max_nn=%u above %d is only supported when it is >= the indexed point count", max_nn, PCC_MAX_K);
         const int th = heap_threads((int)max_nn);
-        PCC_CUDA(cudaFuncSetAttribute(radius_capped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        PCC_TRY(set_heap_smem(radius_capped_kernel));
         radius_capped_kernel<<<nblocks(qs.nq, th), th, (size_t)max_nn * th * sizeof(nkey_t), s>>>(idx->grid(), view_of(qs), r2, ring0(idx, radius), (int)max_nn, d_offsets, keys);
         PCC_LAUNCHED();
         PCC_CUDA(cudaGetLastError());
@@ -773,18 +760,44 @@ int knn_select(pcc_index *idx, const Queries &qs, int k, int32_t *oi, float *od,
 
 using namespace pcc;
 
-static int check_common(pcc_index *idx, void *stream = nullptr) {
-    if (!idx) return fail(PCC_ERR_INVALID, "idx is NULL");
-    if (!idx->built) return fail(PCC_ERR_STATE, "index not built (call pcc_build first)");
-    PCC_CUDA(cudaSetDevice(idx->device));
-    if (!idx->occ_valid) PCC_TRY(rebuild_occupancy(idx, (cudaStream_t)stream));     // first query after pcc_adopt (same rule as pcc_knn.cu)
-    return PCC_OK;
+// The sorted-radius-row consumers (normals, intensity gradient, RIFT, SIFT DoG) after their own checks and input staging: the
+// batch's radius rows sorted by (d2, index) (offsets in idx->out_l, keys in idx->keys64), the output (the caller's pointer, or out_f
+// for PCC_HOST) with the rows of unindexed points pre-filled -- 0xFF bytes (NaN), or (NaN, NaN, NaN, 0) for the gradient -- and
+// launch(offsets, keys, out) when there are queries.  Host inputs are staged in stage4 (free after pcc_build) and sel_params (only
+// used inside the k > 32 kNN selection); the rows touch neither.  A PCC_HOST call returns with its results on the host.
+template <class Launch>
+static int sorted_rows_consumer(pcc_index *idx, const Queries &qs, double radius, void *out, size_t row_bytes, bool fill_nan_w0, int mem, cudaStream_t s,
+                                Launch &&launch) {
+    KernelTimer timer(idx, s);
+    if (!idx->inv_valid) PCC_TRY(rebuild_inverse(idx, s));
+    PCC_TRY(idx->out_l.reserve((size_t)(qs.rows + 1) * 8));
+    int64_t *d_off = idx->out_l.as<int64_t>();
+    PCC_TRY(radius_offsets(idx, qs, radius, 0, d_off, s));
+    int64_t *h = (int64_t *)idx->h_pinned;
+    PCC_CUDA(cudaMemcpyAsync(h, d_off + qs.rows, 8, cudaMemcpyDeviceToHost, s));
+    PCC_CUDA(cudaStreamSynchronize(s));
+    nkey_t *keys = nullptr;
+    PCC_TRY(radius_rows(idx, qs, radius, 0, 1, d_off, h[0], &keys, s));
+    const size_t bytes = (size_t)qs.rows * row_bytes;
+    void *od = nullptr;
+    PCC_TRY(output_rows(idx, out, bytes, mem, &od));
+    if (qs.self && !idx->all_rows_indexed) {
+        if (fill_nan_w0) { fill_f4_kernel<<<nblocks(qs.rows, 256), 256, 0, s>>>((float4 *)od, qs.rows, make_float4(NAN, NAN, NAN, 0.f)); PCC_LAUNCHED(); }
+        else PCC_CUDA(cudaMemsetAsync(od, 0xFF, bytes, s));
+    }
+    if (qs.nq > 0) {
+        launch(d_off, keys, od);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    timer.stop();
+    return deliver_rows(out, od, bytes, mem, s);
 }
 
 extern "C" {
 
 int pcc_radius_count(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, unsigned max_nn, int64_t *offsets, int64_t *total, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(radius >= 0) || !offsets) return fail(PCC_ERR_INVALID, "bad radius / offsets");
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
@@ -804,7 +817,7 @@ int pcc_radius_count(pcc_index *idx, const void *q, int64_t nq, int stride_bytes
 
 int pcc_radius_fill(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, unsigned max_nn, int sorted, const int64_t *offsets,
                     int32_t *out_idx, float *out_d2, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(radius >= 0) || !offsets) return fail(PCC_ERR_INVALID, "bad radius / offsets");
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
@@ -842,95 +855,40 @@ int pcc_radius_fill(pcc_index *idx, const void *q, int64_t nq, int stride_bytes,
 }
 
 int pcc_normals_radius(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float viewpoint[3], float *out, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(radius >= 0)) return fail(PCC_ERR_INVALID, "bad radius");
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
     PCC_TRY(prepare_queries(idx, q, nq, stride_bytes, mem, s, &qs));
     if (qs.rows == 0) return PCC_OK;
     if (!out) return fail(PCC_ERR_INVALID, "output pointer is NULL");
-    if (!idx->inv_valid) PCC_TRY(rebuild_inverse(idx, s));
-    PCC_TRY(idx->out_l.reserve((size_t)(qs.rows + 1) * 8));
-    int64_t *d_off = idx->out_l.as<int64_t>();
-    KernelTimer timer(idx, s);
-    PCC_TRY(radius_offsets(idx, qs, radius, 0, d_off, s));
-    int64_t *h = (int64_t *)idx->h_pinned;
-    PCC_CUDA(cudaMemcpyAsync(h, d_off + qs.rows, 8, cudaMemcpyDeviceToHost, s));
-    PCC_CUDA(cudaStreamSynchronize(s));
-    const int64_t total = h[0];
-    nkey_t *keys = nullptr;
-    PCC_TRY(radius_rows(idx, qs, radius, 0, 1, d_off, total, &keys, s));
-    float4 *od = (float4 *)out;
-    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * 16)); od = idx->out_f.as<float4>(); }
-    if (qs.self && !idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0xFF, (size_t)qs.rows * 16, s));
     const float vx = viewpoint ? viewpoint[0] : 0.f, vy = viewpoint ? viewpoint[1] : 0.f, vz = viewpoint ? viewpoint[2] : 0.f;
-    if (qs.nq > 0) {
-        normals_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), vx, vy, vz, od);
-        PCC_LAUNCHED();
-        PCC_CUDA(cudaGetLastError());
-    }
-    timer.stop();
-    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * 16, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
-    return PCC_OK;
-}
-
-// shared front half of the two descriptor consumers: sorted radius rows of the batch in idx->keys64, offsets in idx->out_l
-static int descriptor_rows(pcc_index *idx, const Queries &qs, double radius, int64_t **d_off_out, nkey_t **keys_out, cudaStream_t s) {
-    if (!idx->inv_valid) PCC_TRY(rebuild_inverse(idx, s));
-    PCC_TRY(idx->out_l.reserve((size_t)(qs.rows + 1) * 8));
-    int64_t *d_off = idx->out_l.as<int64_t>();
-    PCC_TRY(radius_offsets(idx, qs, radius, 0, d_off, s));
-    int64_t *h = (int64_t *)idx->h_pinned;
-    PCC_CUDA(cudaMemcpyAsync(h, d_off + qs.rows, 8, cudaMemcpyDeviceToHost, s));
-    PCC_CUDA(cudaStreamSynchronize(s));
-    *d_off_out = d_off;
-    return radius_rows(idx, qs, radius, 0, 1, d_off, h[0], keys_out, s);
-}
-// host inputs of the descriptor consumers go to device scratch: stage4 is free after pcc_build, sel_params is only used inside
-// the k > 32 kNN selection (the radius rows below touch neither)
-static int stage_in(pcc::Buf &buf, const void *src, size_t bytes, int mem, cudaStream_t s, const void **dev) {
-    if (mem != PCC_HOST) { *dev = src; return PCC_OK; }
-    PCC_TRY(buf.reserve(std::max<size_t>(bytes, 16)));
-    PCC_CUDA(cudaMemcpyAsync(buf.p, src, bytes, cudaMemcpyHostToDevice, s));
-    *dev = buf.p;
-    return PCC_OK;
+    return sorted_rows_consumer(idx, qs, radius, out, 16, false, mem, s, [&](const int64_t *d_off, const nkey_t *keys, void *od) {
+        normals_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), vx, vy, vz, (float4 *)od);
+    });
 }
 
 int pcc_intensity_gradient(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *intensity, const float *normals4,
                            float *out, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(radius >= 0)) return fail(PCC_ERR_INVALID, "bad radius");
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
     PCC_TRY(prepare_queries(idx, q, nq, stride_bytes, mem, s, &qs));
     if (qs.rows == 0) return PCC_OK;
     if (!out || !intensity || !normals4) return fail(PCC_ERR_INVALID, "intensity / normals / output pointer is NULL");
-    const void *d_int = nullptr, *d_nrm = nullptr;
+    const float *d_int = nullptr, *d_nrm = nullptr;
     PCC_TRY(stage_in(idx->stage4, intensity, (size_t)idx->n_input * 4, mem, s, &d_int));
     PCC_TRY(stage_in(idx->sel_params, normals4, (size_t)qs.rows * 16, mem, s, &d_nrm));
-    KernelTimer timer(idx, s);
-    int64_t *d_off = nullptr; nkey_t *keys = nullptr;
-    PCC_TRY(descriptor_rows(idx, qs, radius, &d_off, &keys, s));
-    float4 *od = (float4 *)out;
-    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * 16)); od = idx->out_f.as<float4>(); }
-    if (qs.self && !idx->all_rows_indexed) {
-        fill_f4_kernel<<<nblocks(qs.rows, 256), 256, 0, s>>>(od, qs.rows, make_float4(NAN, NAN, NAN, 0.f));
-        PCC_LAUNCHED();
-    }
-    if (qs.nq > 0) {
-        gradient_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), (const float *)d_int,
-                                                                 (const float4 *)d_nrm, od);
-        PCC_LAUNCHED();
-        PCC_CUDA(cudaGetLastError());
-    }
-    timer.stop();
-    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * 16, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
-    return PCC_OK;
+    return sorted_rows_consumer(idx, qs, radius, out, 16, true, mem, s, [&](const int64_t *d_off, const nkey_t *keys, void *od) {
+        gradient_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), d_int, (const float4 *)d_nrm,
+                                                                 (float4 *)od);
+    });
 }
 
 int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *gradient4, int n_distance_bins, int n_gradient_bins,
              float *out, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(radius >= 0)) return fail(PCC_ERR_INVALID, "bad radius");
     if (n_distance_bins < 1 || n_gradient_bins < 1 || n_distance_bins * n_gradient_bins > 32)
         return fail(PCC_ERR_INVALID, "RIFT bins %d x %d: the histogram holds 1..32 bins (pcl::Histogram<32>)", n_distance_bins, n_gradient_bins);
@@ -939,28 +897,16 @@ int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double
     PCC_TRY(prepare_queries(idx, q, nq, stride_bytes, mem, s, &qs));
     if (qs.rows == 0) return PCC_OK;
     if (!out || !gradient4) return fail(PCC_ERR_INVALID, "gradient / output pointer is NULL");
-    const int nb = n_distance_bins * n_gradient_bins;
-    const void *d_grad = nullptr;
+    const float *d_grad = nullptr;
     PCC_TRY(stage_in(idx->stage4, gradient4, (size_t)idx->n_input * 16, mem, s, &d_grad));
-    KernelTimer timer(idx, s);
-    int64_t *d_off = nullptr; nkey_t *keys = nullptr;
-    PCC_TRY(descriptor_rows(idx, qs, radius, &d_off, &keys, s));
-    float *od = out;
-    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * nb * 4)); od = idx->out_f.as<float>(); }
-    if (qs.self && !idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0xFF, (size_t)qs.rows * nb * 4, s));
-    if (qs.nq > 0) {
+    return sorted_rows_consumer(idx, qs, radius, out, (size_t)n_distance_bins * n_gradient_bins * 4, false, mem, s, [&](const int64_t *d_off, const nkey_t *keys, void *od) {
         rift_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, idx->inv_pos.as<uint32_t>(), (const float4 *)d_grad,
-                                                             (float)radius, n_distance_bins, n_gradient_bins, od);
-        PCC_LAUNCHED();
-        PCC_CUDA(cudaGetLastError());
-    }
-    timer.stop();
-    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * nb * 4, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
-    return PCC_OK;
+                                                             (float)radius, n_distance_bins, n_gradient_bins, (float *)od);
+    });
 }
 
 int pcc_sift_dog(pcc_index *idx, const float *values, const float *scales, int n_scales, float *out, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!scales || n_scales < 2 || n_scales > 16) return fail(PCC_ERR_INVALID, "SIFT scale space of %d scales: 2..16 are supported", n_scales);
     SiftScales sc{};
     for (int i = 0; i < n_scales; ++i) {
@@ -975,27 +921,15 @@ int pcc_sift_dog(pcc_index *idx, const float *values, const float *scales, int n
     PCC_TRY(prepare_queries(idx, nullptr, 0, 16, mem, s, &qs));
     if (qs.rows == 0) return PCC_OK;
     if (!out || !values) return fail(PCC_ERR_INVALID, "values / output pointer is NULL");
-    const int nc = n_scales - 1;
-    const void *d_val = nullptr;
+    const float *d_val = nullptr;
     PCC_TRY(stage_in(idx->stage4, values, (size_t)idx->n_input * 4, mem, s, &d_val));
-    KernelTimer timer(idx, s);
-    int64_t *d_off = nullptr; nkey_t *keys = nullptr;
-    PCC_TRY(descriptor_rows(idx, qs, radius, &d_off, &keys, s));
-    float *od = out;
-    if (mem == PCC_HOST) { PCC_TRY(idx->out_f.reserve((size_t)qs.rows * nc * 4)); od = idx->out_f.as<float>(); }
-    if (!idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(od, 0xFF, (size_t)qs.rows * nc * 4, s));
-    if (qs.nq > 0) {
-        sift_dog_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, (const float *)d_val, sc, n_scales, od);
-        PCC_LAUNCHED();
-        PCC_CUDA(cudaGetLastError());
-    }
-    timer.stop();
-    if (mem == PCC_HOST) { PCC_TRY(copy_out(out, od, (size_t)qs.rows * nc * 4, mem, s)); PCC_CUDA(cudaStreamSynchronize(s)); }
-    return PCC_OK;
+    return sorted_rows_consumer(idx, qs, radius, out, (size_t)(n_scales - 1) * 4, false, mem, s, [&](const int64_t *d_off, const nkey_t *keys, void *od) {
+        sift_dog_rows_kernel<<<nblocks(qs.nq, 128), 128, 0, s>>>(idx->grid(), view_of(qs), d_off, keys, d_val, sc, n_scales, (float *)od);
+    });
 }
 
 int pcc_first_within(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double thr, int32_t *out, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(thr >= 0) || !q) return fail(PCC_ERR_INVALID, "bad threshold / queries");
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
@@ -1064,7 +998,7 @@ static int ece_finish(pcc_index *idx, uint32_t *parent, int64_t min_size, int64_
 
 int pcc_euclidean_labels(pcc_index *idx, double tolerance, int64_t min_size, int64_t max_size, int32_t *labels, int64_t *n_clusters, int64_t *sizes,
                          int64_t sizes_cap, int mem, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(tolerance >= 0) || !labels || !n_clusters) return fail(PCC_ERR_INVALID, "bad tolerance / outputs");
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t n = idx->n_indexed;
@@ -1085,13 +1019,13 @@ int pcc_euclidean_labels(pcc_index *idx, double tolerance, int64_t min_size, int
 
 // ---- sharded clustering (SURVEY.md section 8e): parent forests over SORTED positions, device memory only ----
 int pcc_ece_init(pcc_index *idx, uint32_t *parent, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!parent) return fail(PCC_ERR_INVALID, "parent is NULL");
     if (idx->n_indexed > 0) { iota_kernel<<<nblocks(idx->n_indexed, 256), 256, 0, (cudaStream_t)stream>>>(parent, idx->n_indexed); PCC_LAUNCHED(); PCC_CUDA(cudaGetLastError()); }
     return PCC_OK;
 }
 int pcc_ece_link_range(pcc_index *idx, double tolerance, int64_t begin, int64_t end, uint32_t *parent, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!(tolerance >= 0) || !parent || begin < 0 || end > idx->n_indexed || begin > end) return fail(PCC_ERR_INVALID, "bad range [%lld, %lld) of %lld", (long long)begin, (long long)end, (long long)idx->n_indexed);
     if (end > begin) {
         ece_link_range_kernel<<<nblocks(end - begin, 128), 128, 0, (cudaStream_t)stream>>>(idx->grid(), (float)(tolerance * tolerance), ring0(idx, tolerance), (uint32_t)begin, (uint32_t)end, parent);
@@ -1100,7 +1034,7 @@ int pcc_ece_link_range(pcc_index *idx, double tolerance, int64_t begin, int64_t 
     return PCC_OK;
 }
 int pcc_ece_absorb(pcc_index *idx, const uint32_t *other, uint32_t *parent, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!other || !parent) return fail(PCC_ERR_INVALID, "NULL forest");
     if (idx->n_indexed > 0) {
         ece_absorb_kernel<<<nblocks(idx->n_indexed, 256), 256, 0, (cudaStream_t)stream>>>((uint32_t)idx->n_indexed, other, parent); PCC_LAUNCHED();
@@ -1110,7 +1044,7 @@ int pcc_ece_absorb(pcc_index *idx, const uint32_t *other, uint32_t *parent, void
     return PCC_OK;
 }
 int pcc_ece_finish(pcc_index *idx, uint32_t *parent, int64_t min_size, int64_t max_size, int32_t *labels, int64_t *n_clusters, int64_t *sizes, int64_t sizes_cap, void *stream) {
-    PCC_TRY(check_common(idx));
+    PCC_TRY(check_index(idx, stream));
     if (!parent || !labels || !n_clusters) return fail(PCC_ERR_INVALID, "NULL argument");
     *n_clusters = 0;
     if (idx->n_input == 0) return PCC_OK;

@@ -13,8 +13,6 @@
 
 namespace pcc {
 
-static inline unsigned nblocks(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
-
 static constexpr int kSiftK = 25;          // findScaleSpaceExtrema: const int k = 25
 static constexpr int kSiftMaxCols = 15;    // DoG columns: nr_scales_per_octave + 2 <= 15
 
@@ -101,23 +99,17 @@ extern "C" {
 
 int pcc_sift_extrema(pcc_index *idx, const float *dog, int n_cols, float min_contrast, int32_t *out_row, int32_t *out_col, int64_t cap, int64_t *n_found,
                      int mem, void *stream) {
-    if (!idx) return fail(PCC_ERR_INVALID, "idx is NULL");
-    if (!idx->built) return fail(PCC_ERR_STATE, "index not built (call pcc_build first)");
+    PCC_TRY(check_index(idx, stream));
     if (n_cols < 1 || n_cols > kSiftMaxCols) return fail(PCC_ERR_INVALID, "SIFT DoG of %d columns: 1..%d are supported", n_cols, kSiftMaxCols);
     if (!n_found || cap < 0 || (cap > 0 && (!out_row || !out_col)) || !(min_contrast >= 0.f)) return fail(PCC_ERR_INVALID, "bad arguments");
-    PCC_CUDA(cudaSetDevice(idx->device));
     cudaStream_t s = (cudaStream_t)stream;
     *n_found = 0;
     const int64_t n = idx->n_input, m = n * n_cols;
     if (n == 0) return PCC_OK;
     if (!dog) return fail(PCC_ERR_INVALID, "dog is NULL");
     if (m >= (1ll << 31) - 1) return fail(PCC_ERR_INVALID, "%lld DoG entries exceed the 32-bit scan", (long long)m);
-    const float *d_dog = dog;
-    if (mem == PCC_HOST) {
-        PCC_TRY(idx->sift_in.reserve((size_t)m * 4));
-        PCC_CUDA(cudaMemcpyAsync(idx->sift_in.p, dog, (size_t)m * 4, cudaMemcpyHostToDevice, s));
-        d_dog = idx->sift_in.as<float>();
-    }
+    const float *d_dog = nullptr;
+    PCC_TRY(stage_in(idx->sift_in, dog, (size_t)m * 4, mem, s, &d_dog));
     const int k = (int)std::min<int64_t>(kSiftK, std::max<int64_t>(idx->n_indexed, 1));       // nearestKSearch returns min(k, size) rows
     PCC_TRY(idx->sift_nbr.reserve((size_t)n * k * 4));
     PCC_TRY(idx->sift_d2.reserve((size_t)n * k * 4));

@@ -15,8 +15,6 @@
 
 namespace pcc {
 
-static inline unsigned nblocks(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
-
 struct VoxelParams { float inv[3]; int min_b[3]; int mul[3]; };
 
 __device__ __forceinline__ int f2ord_v(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7FFFFFFF; }
@@ -109,15 +107,10 @@ extern "C" int pcc_voxel_grid(pcc_index *idx, const void *pts, int64_t n, int st
     cudaStream_t s = (cudaStream_t)stream;
     *n_out = 0;
     if (n == 0) return PCC_OK;
-    const uint8_t *raw = (const uint8_t *)pts;
+    const uint8_t *raw = nullptr;
+    PCC_TRY(stage_in(idx->raw, (const uint8_t *)pts, (size_t)n * stride_bytes, mem, s, &raw));
     uint8_t *d_out = (uint8_t *)out;
-    if (mem == PCC_HOST) {
-        PCC_TRY(idx->raw.reserve((size_t)n * stride_bytes));
-        PCC_CUDA(cudaMemcpyAsync(idx->raw.p, pts, (size_t)n * stride_bytes, cudaMemcpyHostToDevice, s));
-        raw = idx->raw.as<uint8_t>();
-        PCC_TRY(idx->stage4.reserve((size_t)n * stride_bytes));
-        d_out = idx->stage4.as<uint8_t>();
-    }
+    if (mem == PCC_HOST) { PCC_TRY(idx->stage4.reserve((size_t)n * stride_bytes)); d_out = idx->stage4.as<uint8_t>(); }
     // 1. bounding box of the finite points
     int *h = (int *)idx->h_pinned;
     PCC_TRY(idx->keys64.reserve(256));
