@@ -580,6 +580,56 @@ class SIFTKeypoint {
     int nr_octaves_ = 5, nr_scales_per_octave_ = 5;
 };
 
+// SIFTKeypoint over every cluster of a cloud in one call (pcc_sift_keypoints_batched), as processRIFTwithSIFT runs it per cluster
+// (src/comparator.cpp:1228, 1264): compute fills out[c] with exactly what SIFTKeypoint::compute returns on cluster c alone, and, when
+// `snap` is given, (*snap)[c] with the cluster-local row of the first point of cluster c within snap_threshold of each keypoint
+// (-1 if none; src/comparator.cpp:696-713).  Clusters are copied into one concatenated cloud for the call.
+template <typename PointT>
+class SIFTKeypointBatched {
+  public:
+    explicit SIFTKeypointBatched(int device = 0) { check(pcc_create(device, &ws_)); }
+    ~SIFTKeypointBatched() { pcc_destroy(ws_); }
+    SIFTKeypointBatched(const SIFTKeypointBatched &) = delete;
+    SIFTKeypointBatched &operator=(const SIFTKeypointBatched &) = delete;
+    void setInputClouds(const std::vector<typename search::GridSearch<PointT>::PointCloudConstPtr> &clouds) { inputs_ = clouds; }
+    void setScales(float min_scale, int nr_octaves, int nr_scales_per_octave) { min_scale_ = min_scale; nr_octaves_ = nr_octaves; nr_scales_per_octave_ = nr_scales_per_octave; }
+    void setMinimumContrast(float min_contrast) { min_contrast_ = min_contrast; }
+    void compute(std::vector<std::vector<PointWithScale> > &out, std::vector<std::vector<int> > *snap = nullptr, double snap_threshold = 0.05) {
+        std::vector<PointT> all;
+        std::vector<int64_t> off(1, 0);
+        for (const auto &c : inputs_) {
+            if (!c) throw Error("SIFTKeypointBatched: null input cloud");
+            all.insert(all.end(), c->points.begin(), c->points.end());
+            off.push_back((int64_t)all.size());
+        }
+        const int64_t n_clouds = (int64_t)inputs_.size();
+        std::vector<int64_t> kp_off(off.size());
+        std::vector<PointWithScale> kp;
+        std::vector<int32_t> sn;
+        int64_t cap = std::max<int64_t>((int64_t)all.size(), 1);
+        for (;;) {                                   // the keypoint count is known after the call: retry once with room for all
+            kp.resize((size_t)cap);
+            if (snap) sn.resize((size_t)cap);
+            check(pcc_sift_keypoints_batched(ws_, all.data(), (int64_t)all.size(), (int)sizeof(PointT), (int)offsetof(PointT, rgb), off.data(), n_clouds,
+                                             min_scale_, nr_octaves_, nr_scales_per_octave_, min_contrast_, snap_threshold,
+                                             reinterpret_cast<float *>(kp.data()), snap ? sn.data() : nullptr, cap, kp_off.data(), PCC_HOST, nullptr));
+            if (kp_off.back() <= cap) break;
+            cap = kp_off.back();
+        }
+        out.assign((size_t)n_clouds, std::vector<PointWithScale>());
+        if (snap) snap->assign((size_t)n_clouds, std::vector<int>());
+        for (int64_t c = 0; c < n_clouds; ++c) {
+            out[c].assign(kp.begin() + kp_off[c], kp.begin() + kp_off[c + 1]);
+            if (snap) (*snap)[c].assign(sn.begin() + kp_off[c], sn.begin() + kp_off[c + 1]);
+        }
+    }
+  private:
+    pcc_index *ws_ = nullptr;
+    std::vector<typename search::GridSearch<PointT>::PointCloudConstPtr> inputs_;
+    float min_scale_ = 0.005f, min_contrast_ = 0.001f;
+    int nr_octaves_ = 5, nr_scales_per_octave_ = 5;
+};
+
 // matchRIFTFeaturesKnn (src/comparator.cpp:560-588): KdTreeFLANN<Histogram<32>> over descriptors1, nearestKSearch(k = 1) for every
 // descriptor of descriptors2, kept when the squared distance is < 0.05.  The returned vector starts with one 0, as the reference's
 // `std::vector<int> correspondence(1)` does (its callers use size()).  HistT is any POD whose first floats are the histogram

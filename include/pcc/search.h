@@ -137,6 +137,19 @@ int pcc_sift_extrema(pcc_index *idx, const float *dog, int n_cols, float min_con
  * `idx` is the workspace: the call rebuilds it per octave and leaves it indexing the last octave's grid. */
 int pcc_sift_keypoints(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, int rgb_offset_bytes, float min_scale, int nr_octaves,
                        int nr_scales_per_octave, float min_contrast, float *out4, int64_t cap, int64_t *n_keypoints, int mem, void *stream);
+/* pcc_sift_keypoints, then pcc_first_within, on every cluster of a concatenated cloud in one call (processRIFTwithSIFT's per-cluster
+ * processSift + snap, src/comparator.cpp:435-469, 696-713).  Cluster c is rows [cloud_offsets[c], cloud_offsets[c+1]) of pts (row
+ * layout as pcc_sift_keypoints); cloud_offsets (HOST, n_clouds + 1 entries) starts at 0, ends at n and never decreases, empty clusters
+ * allowed.  out4 gets every cluster's pcc_sift_keypoints rows, bit for bit, concatenated in cluster order -- (cluster, octave, point,
+ * column) order, at most `cap` rows; kp_offsets (HOST, n_clouds + 1) always gets the full layout, kp_offsets[n_clouds] = total.
+ * snap (may be NULL) gets one int32 per written row: the cluster-LOCAL row of the lowest-index point of the keypoint's own cluster
+ * with sqrt(double d^2) < snap_threshold, or -1.  The octave loop runs once for the batch; a cluster leaves it at the first octave
+ * whose VoxelGrid result has fewer than 25 points.  Host round trips depend on the octave count, not on n_clouds (<= 2^24).
+ * `idx` is the workspace: after the call it indexes the concatenated input (cell snap_threshold) when snap is non-NULL and a row was
+ * written, else the union of the clusters' last octave clouds. */
+int pcc_sift_keypoints_batched(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, int rgb_offset_bytes, const int64_t *cloud_offsets,
+                               int64_t n_clouds, float min_scale, int nr_octaves, int nr_scales_per_octave, float min_contrast, double snap_threshold,
+                               float *out4, int32_t *snap, int64_t cap, int64_t *kp_offsets, int mem, void *stream);
 
 /* CorrespondenceEstimation::determineCorrespondences + the sums TransformationEstimationSVD needs
  * (src/comparator.cpp:1091-1096) [up].  Each source point is first moved by the row-major 4x4 `T_apply`

@@ -57,6 +57,14 @@ __device__ __forceinline__ int64_t rows_query(const Grid &g, const QueryView &v,
     uint32_t qi = v.order ? __ldg(v.order + t) : (uint32_t)t; float4 p = __ldg(v.q + qi); x = p.x; y = p.y; z = p.z; return qi;
 }
 
+// segment of row i of a concatenation whose segment c is rows [off[c], off[c+1]) (off[0] = 0 <= i < off[n_seg]): the last c with
+// off[c] <= i, so empty segments, which share their offset with the next one, never match
+__device__ __forceinline__ uint32_t segment_of(const int64_t *__restrict__ off, int n_seg, int64_t i) {
+    int lo = 0, hi = n_seg;
+    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (__ldg(off + mid) <= i) lo = mid; else hi = mid; }
+    return (uint32_t)lo;
+}
+
 struct QueryCell {
     float ux, uy, uz;
     int cx, cy, cz;

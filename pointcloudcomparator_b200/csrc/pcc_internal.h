@@ -72,6 +72,9 @@ struct pcc_index {
     pcc::Buf raw, stage4, cellrank, qbuf, qkeys, qkeys2, qperm, qperm2, cub_tmp, out_i, out_f, out_l, keys64, keys64b, misc, parent, inv_pos, sel_params, icp_prior, calib;
     // pcc_sift_*: the octave clouds (ping-pong, float4 x, y, z, packed rgb) live outside the scratch pcc_voxel_grid and pcc_build reuse
     pcc::Buf sift_cloud[2], sift_val, sift_dog, sift_in, sift_nbr, sift_d2, sift_flag, sift_pos, sift_row, sift_col, sift_kp;
+    // pcc_sift_keypoints_batched: segment label per sorted position of the current grid (segment_labels), the octave's segment
+    // offsets, per-segment tables, per-row segment labels of the segmented VoxelGrid and the keypoints staged across octaves
+    pcc::Buf seg_label, seg_off, sift_tab, sift_lab, sift_stage;
     uint64_t grid_gen = 0;     // bumped by pcc_build / pcc_adopt
     void *comm = nullptr;      // ncclComm_t handed to pcc_comm_init (not owned); rank / world of this process in it
     int comm_rank = 0, comm_world = 1;
@@ -163,6 +166,23 @@ int rebuild_inverse(pcc_index *idx, cudaStream_t s);
 int comm_allreduce_f64(pcc_index *idx, double *d_buf, int n, cudaStream_t s);   // pcc_comm.cu; no-op without a communicator
 // k > 32: neighbours by selection (pcc_radius.cu); rows are sorted by (d2, index), oi / od are device pointers
 int knn_select(pcc_index *idx, const Queries &qs, int k, int32_t *oi, float *od, cudaStream_t s);
+// ---- segmented clouds: segment c is rows [off[c], off[c+1]) of a concatenation (pcc_sift_keypoints_batched) ----
+// idx->seg_label[sorted position] = segment of the point's original row; d_off is a device array of n_seg + 1 offsets
+int segment_labels(pcc_index *idx, const int64_t *d_off, int n_seg, cudaStream_t s);
+// the indexed cloud's own radius rows with neighbours of the query's segment only, sorted by (d2, index): offsets (n_input + 1,
+// in idx->out_l) and keys (idx->keys64); rows of unindexed points are empty
+int segmented_sorted_rows(pcc_index *idx, const uint32_t *seg, double radius, const int64_t **d_off, const nkey_t **keys, cudaStream_t s);
+// pcc_sift_dog over segmented_sorted_rows (device pointers, no checks); rows of unindexed points are NaN
+int sift_dog_segmented(pcc_index *idx, const uint32_t *seg, const float *values, const float *scales, int n_scales, float *out, cudaStream_t s);
+// pcc_first_within restricted to the query's segment: query t belongs to segment segment_of(d_qoff, t), the indexed points carry
+// their segment in seg, and out[t] is relative to that segment's first row (d_poff).  q, d_qoff, d_poff and out are device pointers.
+int first_within_segmented(pcc_index *idx, const uint32_t *seg, const float4 *q, int64_t nq, const int64_t *d_qoff, const int64_t *d_poff, int n_seg,
+                           double thr, int32_t *out, cudaStream_t s);
+// VoxelGrid (leaf in every axis, rgb averaged) of every segment of a float4 (x, y, z, rgb word) cloud, each segment with its own
+// bounding box, exactly as pcc_voxel_grid on that segment alone.  in_off / out_off are host arrays of n_seg + 1 offsets.  A
+// segment whose result has fewer than min_rows rows is dropped (no rows in `out`); the others are written in segment order.
+int segmented_voxel_grid(pcc_index *idx, const float4 *in, const int64_t *in_off, int n_seg, float leaf, int64_t min_rows, float4 *out, int64_t *out_off,
+                         cudaStream_t s);
 struct KernelTimer {
     pcc_index *idx; cudaStream_t s;
     KernelTimer(pcc_index *i, cudaStream_t st) : idx(i), s(st) { if (idx->timing) cudaEventRecord(idx->ev0, s); }

@@ -539,6 +539,54 @@ __global__ void __launch_bounds__(128) first_within_kernel(Grid g, QueryView v, 
     out[qi] = best == INT_MAX ? -1 : best;
 }
 
+// ---- segmented clouds: neighbours only from the query's own segment (seg[sorted position]) ----
+__global__ void segment_label_kernel(const float4 *__restrict__ pts, int64_t n, const int64_t *__restrict__ off, int n_seg, uint32_t *__restrict__ seg) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n) seg[t] = segment_of(off, n_seg, __float_as_int(__ldg(pts + t).w));
+}
+// radius_count_kernel / radius_fill_kernel for the indexed cloud's own rows, admitting a neighbour when its segment is the query's
+__global__ void __launch_bounds__(128) seg_radius_count_kernel(Grid g, const uint32_t *__restrict__ seg, float r2, int R0, int64_t *__restrict__ counts) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= g.n) return;
+    const float4 q = __ldg(g.pts + t);
+    const uint32_t sq = __ldg(seg + t);
+    unsigned n = 0;
+    radius_visit(g, q.x, q.y, q.z, r2, R0, [&](uint32_t pos, float4, float) { if (__ldg(seg + pos) == sq) ++n; });
+    counts[__float_as_int(q.w)] = n;
+}
+__global__ void __launch_bounds__(128) seg_radius_fill_kernel(Grid g, const uint32_t *__restrict__ seg, float r2, int R0, const int64_t *__restrict__ offsets,
+                                                              nkey_t *__restrict__ keys) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= g.n) return;
+    const float4 q = __ldg(g.pts + t);
+    const uint32_t sq = __ldg(seg + t);
+    nkey_t *o = keys + offsets[__float_as_int(q.w)];
+    radius_visit(g, q.x, q.y, q.z, r2, R0, [&](uint32_t pos, float4 p, float d2) { if (__ldg(seg + pos) == sq) *o++ = make_key(d2, __float_as_uint(p.w)); });
+}
+// first_within_kernel restricted to the query's segment (segment_of(qoff, t)); the answer is relative to the segment's first row
+__global__ void __launch_bounds__(128) first_within_seg_kernel(Grid g, const uint32_t *__restrict__ seg, const float4 *__restrict__ qp, int64_t nq,
+                                                               const int64_t *__restrict__ qoff, const int64_t *__restrict__ poff, int n_seg, double thr,
+                                                               float r2_cover, int R0, int32_t *__restrict__ out) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nq) return;
+    const float4 q = __ldg(qp + t);
+    const uint32_t sq = segment_of(qoff, n_seg, t);
+    int32_t best = INT_MAX;
+    if (finite3(q.x, q.y, q.z) && g.n > 0) {
+        const QueryCell c = locate(g, q.x, q.y, q.z);
+        int Rin = -1, R = R0;
+        for (;;) {
+            scan_shell(g, c, Rin, R, [&](uint32_t pos, float4 p) {
+                const double dx = (double)(q.x - p.x), dy = (double)(q.y - p.y), dz = (double)(q.z - p.z);
+                if (__ldg(seg + pos) == sq && sqrt(dx * dx + dy * dy + dz * dz) < thr) best = min(best, __float_as_int(p.w));
+            });
+            if (covered_d2(g, c, R) >= r2_cover) break;
+            Rin = R; ++R;
+        }
+    }
+    out[t] = best == INT_MAX ? -1 : best - (int32_t)__ldg(poff + sq);
+}
+
 // ---- EuclideanClusterExtraction: lock-free union-find over sorted positions ----
 // Loads bypass L1 (__ldcg) so a root that another SM has just hooked is seen in L2; a stale value is still
 // an ancestor in the same set, so following it is safe, and the CAS below is the only way a root changes.
@@ -765,6 +813,73 @@ using namespace pcc;
 // for PCC_HOST) with the rows of unindexed points pre-filled -- 0xFF bytes (NaN), or (NaN, NaN, NaN, 0) for the gradient -- and
 // launch(offsets, keys, out) when there are queries.  Host inputs are staged in stage4 (free after pcc_build) and sel_params (only
 // used inside the k > 32 kNN selection); the rows touch neither.  A PCC_HOST call returns with its results on the host.
+static SiftScales sift_scale_table(const float *scales, int n_scales) {
+    SiftScales sc{};
+    for (int i = 0; i < n_scales; ++i) {
+        sc.sigma_sqr[i] = powf(scales[i], 2.0f);                 // computeScaleSpace: sigma_sqr = powf (scales[i_scale], 2.0f)
+        sc.cutoff[i] = 9 * sc.sigma_sqr[i];                      // if (dist_sqr <= 9*sigma_sqr)
+    }
+    return sc;
+}
+static double sift_radius(const float *scales, int n_scales) { return (double)(3.0f * scales[n_scales - 1]); }   // max_radius = 3.0f * scales.back (), a float handed to radiusSearch
+
+int pcc::segment_labels(pcc_index *idx, const int64_t *d_off, int n_seg, cudaStream_t s) {
+    PCC_TRY(idx->seg_label.reserve((size_t)std::max<int64_t>(idx->n_indexed, 1) * 4));
+    if (idx->n_indexed > 0) {
+        segment_label_kernel<<<nblocks(idx->n_indexed, 256), 256, 0, s>>>(idx->pts.as<float4>(), idx->n_indexed, d_off, n_seg, idx->seg_label.as<uint32_t>());
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    return PCC_OK;
+}
+int pcc::segmented_sorted_rows(pcc_index *idx, const uint32_t *seg, double radius, const int64_t **d_off_out, const nkey_t **keys_out, cudaStream_t s) {
+    const int64_t rows = idx->n_input, n = idx->n_indexed;
+    const float r2 = (float)(radius * radius);
+    PCC_TRY(idx->out_l.reserve((size_t)(rows + 1) * 8));
+    int64_t *d_off = idx->out_l.as<int64_t>();
+    PCC_CUDA(cudaMemsetAsync(d_off, 0, (size_t)(rows + 1) * sizeof(int64_t), s));
+    if (n > 0) { seg_radius_count_kernel<<<nblocks(n, 128), 128, 0, s>>>(idx->grid(), seg, r2, ring0(idx, radius), d_off); PCC_LAUNCHED(); PCC_CUDA(cudaGetLastError()); }
+    size_t tmp = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp, d_off, d_off, (int)(rows + 1), s);
+    PCC_TRY(idx->cub_tmp.reserve(tmp));
+    PCC_CUDA(cub::DeviceScan::ExclusiveSum(idx->cub_tmp.p, tmp, d_off, d_off, (int)(rows + 1), s));
+    g_launches += 2;
+    int64_t *h = (int64_t *)idx->h_pinned;
+    PCC_CUDA(cudaMemcpyAsync(h, d_off + rows, 8, cudaMemcpyDeviceToHost, s));
+    PCC_CUDA(cudaStreamSynchronize(s));
+    const int64_t total = h[0];
+    PCC_TRY(idx->keys64.reserve((size_t)std::max<int64_t>(total, 1) * sizeof(nkey_t)));
+    nkey_t *keys = idx->keys64.as<nkey_t>();
+    *d_off_out = d_off; *keys_out = keys;
+    if (total == 0) return PCC_OK;
+    seg_radius_fill_kernel<<<nblocks(n, 128), 128, 0, s>>>(idx->grid(), seg, r2, ring0(idx, radius), d_off, keys);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    return sort_csr_rows(idx, rows, d_off, total, keys, s);
+}
+int pcc::sift_dog_segmented(pcc_index *idx, const uint32_t *seg, const float *values, const float *scales, int n_scales, float *out, cudaStream_t s) {
+    const SiftScales sc = sift_scale_table(scales, n_scales);
+    const int64_t *d_off = nullptr; const nkey_t *keys = nullptr;
+    PCC_TRY(segmented_sorted_rows(idx, seg, sift_radius(scales, n_scales), &d_off, &keys, s));
+    if (!idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(out, 0xFF, (size_t)idx->n_input * (n_scales - 1) * 4, s));
+    if (idx->n_indexed > 0) {
+        const QueryView v{nullptr, nullptr, idx->n_indexed, true};
+        sift_dog_rows_kernel<<<nblocks(idx->n_indexed, 128), 128, 0, s>>>(idx->grid(), v, d_off, keys, values, sc, n_scales, out);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    return PCC_OK;
+}
+int pcc::first_within_segmented(pcc_index *idx, const uint32_t *seg, const float4 *q, int64_t nq, const int64_t *d_qoff, const int64_t *d_poff, int n_seg,
+                                double thr, int32_t *out, cudaStream_t s) {
+    if (nq == 0) return PCC_OK;
+    const float r2_cover = (float)(thr * thr * (1.0 + 1e-5));       // as pcc_first_within
+    first_within_seg_kernel<<<nblocks(nq, 128), 128, 0, s>>>(idx->grid(), seg, q, nq, d_qoff, d_poff, n_seg, thr, r2_cover, ring0(idx, thr), out);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    return PCC_OK;
+}
+
 template <class Launch>
 static int sorted_rows_consumer(pcc_index *idx, const Queries &qs, double radius, void *out, size_t row_bytes, bool fill_nan_w0, int mem, cudaStream_t s,
                                 Launch &&launch) {
@@ -908,14 +1023,12 @@ int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double
 int pcc_sift_dog(pcc_index *idx, const float *values, const float *scales, int n_scales, float *out, int mem, void *stream) {
     PCC_TRY(check_index(idx, stream));
     if (!scales || n_scales < 2 || n_scales > 16) return fail(PCC_ERR_INVALID, "SIFT scale space of %d scales: 2..16 are supported", n_scales);
-    SiftScales sc{};
     for (int i = 0; i < n_scales; ++i) {
         if (!(scales[i] > 0.f) || !std::isfinite(scales[i]) || (i > 0 && !(scales[i] >= scales[i - 1])))
             return fail(PCC_ERR_INVALID, "SIFT scales must be positive, finite and ascending (scale %d = %g)", i, (double)scales[i]);
-        sc.sigma_sqr[i] = powf(scales[i], 2.0f);                 // computeScaleSpace: sigma_sqr = powf (scales[i_scale], 2.0f)
-        sc.cutoff[i] = 9 * sc.sigma_sqr[i];                      // if (dist_sqr <= 9*sigma_sqr)
     }
-    const double radius = (double)(3.0f * scales[n_scales - 1]);      // max_radius = 3.0f * scales.back (), a float handed to radiusSearch
+    const SiftScales sc = sift_scale_table(scales, n_scales);
+    const double radius = sift_radius(scales, n_scales);
     cudaStream_t s = (cudaStream_t)stream;
     Queries qs;
     PCC_TRY(prepare_queries(idx, nullptr, 0, 16, mem, s, &qs));

@@ -512,6 +512,62 @@ def process_sift(xyz, rgb, snap_threshold: float = 0.05, device: int = 0, **sift
     return kp, s.firstWithin(np.ascontiguousarray(kp[:, :3]), snap_threshold)
 
 
+def _sift_batched(xyz, rgb, offsets, snap_threshold, min_scale, nr_octaves, nr_scales_per_octave, min_contrast, device):
+    """pcc_sift_keypoints_batched over the clusters [offsets[c], offsets[c+1]) of xyz: numpy inputs go through PCC_HOST, a CUDA
+    tensor xyz through PCC_DEVICE on the current stream.  Returns (keypoints [m, 4], kp_offsets int64 [n_clouds + 1], snap or None)."""
+    off = np.ascontiguousarray(np.asarray(offsets), np.int64)
+    n_clouds = off.shape[0] - 1
+    kp_off = np.zeros(max(n_clouds, 0) + 1, np.int64)
+    want_snap = snap_threshold is not None
+    if _is_cuda(xyz):
+        dev = xyz.device
+        c = torch.as_tensor(np.asarray(rgb.cpu().numpy() if _is_cuda(rgb) else rgb).reshape(-1, 3).astype(np.int32), device=dev)
+        rows = torch.empty((xyz.shape[0], 4), dtype=torch.float32, device=dev)
+        rows[:, :3] = xyz[:, :3]
+        rows[:, 3] = ((c[:, 0] << 16) | (c[:, 1] << 8) | c[:, 2]).view(torch.float32)
+        ptr, n, mem = rows.data_ptr(), rows.shape[0], DEVICE
+        alloc = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)          # noqa: E731
+        f32, i32 = torch.float32, torch.int32
+    else:
+        rows = _sift_rows(xyz, rgb)
+        ptr, n, mem = rows.ctypes.data, rows.shape[0], HOST
+        alloc = lambda shape, dt: np.empty(shape, dt)                                 # noqa: E731
+        f32, i32 = np.float32, np.int32
+    L = _lib.lib()
+    ws = GridSearch(device)
+    cap = max(n, 1)
+    while True:
+        out = alloc((cap, 4), f32)
+        snap = alloc((cap,), i32) if want_snap else None
+        op = out.data_ptr() if mem == DEVICE else out.ctypes.data
+        sp = None if snap is None else (snap.data_ptr() if mem == DEVICE else snap.ctypes.data)
+        check(L.pcc_sift_keypoints_batched(ws._h, ptr, n, 16, 12, off.ctypes.data, n_clouds, float(min_scale), int(nr_octaves), int(nr_scales_per_octave),
+                                           float(min_contrast), float(snap_threshold if want_snap else 0.0), op, sp, cap, kp_off.ctypes.data, mem,
+                                           _stream(ws.device)))
+        total = int(kp_off[-1])
+        if total <= cap:
+            break
+        cap = total
+    return out[:total], kp_off, (None if snap is None else snap[:total])
+
+
+def sift_keypoints_batched(xyz, rgb, offsets, min_scale: float = 0.005, nr_octaves: int = 5, nr_scales_per_octave: int = 5, min_contrast: float = 0.001,
+                           device: int = 0):
+    """sift_keypoints on every cluster [offsets[c], offsets[c+1]) of xyz / rgb in one pcc_sift_keypoints_batched call: returns
+    (keypoints float32 [m, 4], kp_offsets int64 [n_clouds + 1]); keypoints[kp_offsets[c]:kp_offsets[c+1]] is sift_keypoints of cluster c,
+    bit for bit.  A CUDA tensor xyz keeps the call and its outputs in device memory."""
+    kp, kp_off, _ = _sift_batched(xyz, rgb, offsets, None, min_scale, nr_octaves, nr_scales_per_octave, min_contrast, device)
+    return kp, kp_off
+
+
+def process_sift_batched(xyz, rgb, offsets, snap_threshold: float = 0.05, device: int = 0, **sift_kw):
+    """process_sift on every cluster of xyz / rgb in one call: (keypoints [m, 4], kp_offsets int64 [n_clouds + 1], snap int32 [m]); snap
+    holds cluster-LOCAL rows (the lowest-index point of the keypoint's own cluster within snap_threshold, -1 if none)."""
+    kw = dict(min_scale=0.005, nr_octaves=5, nr_scales_per_octave=5, min_contrast=0.001)
+    kw.update(sift_kw)
+    return _sift_batched(xyz, rgb, offsets, float(snap_threshold), kw["min_scale"], kw["nr_octaves"], kw["nr_scales_per_octave"], kw["min_contrast"], device)
+
+
 def umeyama_from_sums(sums, count: int):
     T = (C.c_float * 16)()
     s = (C.c_double * 16)(*[float(v) for v in sums])
