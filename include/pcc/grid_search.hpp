@@ -18,6 +18,7 @@
 //   pcc::RegionGrowing               <- pcl::RegionGrowing               (src/segmentation.cpp:249-271)
 //   pcc::IntensityGradientEstimation <- pcl::IntensityGradientEstimation (src/comparator.cpp:649-656)
 //   pcc::RIFTEstimation              <- pcl::RIFTEstimation              (src/comparator.cpp:659-673)
+//   pcc::processRIFTBatched          <- processRIFT on every cluster     (src/comparator.cpp:590-684, 1224-1366)
 // There is no CPU fallback: a failing CUDA call throws pcc::Error.
 #ifndef PCC_GRID_SEARCH_HPP_
 #define PCC_GRID_SEARCH_HPP_
@@ -629,6 +630,47 @@ class SIFTKeypointBatched {
     float min_scale_ = 0.005f, min_contrast_ = 0.001f;
     int nr_octaves_ = 5, nr_scales_per_octave_ = 5;
 };
+
+// processRIFT (src/comparator.cpp:590-684) on every cluster in one call (pcc_rift_batched), as computeSimilarity runs it per cluster:
+// descriptors[c] and kept_rows[c] are exactly what cluster c alone gets from NormalEstimation(radius) -> drop the NaN normals ->
+// IntensityGradientEstimation -> RIFTEstimation -> drop the rows with a non-finite bin.  kept_rows[c] are rows of cluster c; bins beyond
+// nd * ng stay 0.  Intensity is rgbToIntensity of each point's colour, so PointT needs PCL's r, g, b members.  Clusters are copied into
+// one concatenated cloud for the call.
+template <typename PointT>
+inline void processRIFTBatched(const std::vector<typename search::GridSearch<PointT>::PointCloudConstPtr> &clusters,
+                               std::vector<std::vector<Histogram32> > &descriptors, std::vector<std::vector<int> > &kept_rows, double normal_radius = 0.03,
+                               double gradient_radius = 0.03, double rift_radius = 0.05, int nr_distance_bins = 4, int nr_gradient_bins = 8, int device = 0) {
+    std::vector<PointT> all;
+    std::vector<float> inten;
+    std::vector<int64_t> off(1, 0);
+    for (const auto &c : clusters) {
+        if (!c) throw Error("processRIFTBatched: null input cloud");
+        for (const PointT &p : c->points) { all.push_back(p); inten.push_back(rgbToIntensity(p.r, p.g, p.b)); }
+        off.push_back((int64_t)all.size());
+    }
+    const int64_t n_clouds = (int64_t)clusters.size(), n = (int64_t)all.size();
+    const int nb = nr_distance_bins * nr_gradient_bins;
+    std::vector<int64_t> desc_off(off.size());
+    std::vector<float> flat((size_t)std::max<int64_t>(n, 1) * (size_t)std::max(nb, 1));
+    std::vector<int32_t> rows((size_t)std::max<int64_t>(n, 1));
+    pcc_index *ws = nullptr;
+    check(pcc_create(device, &ws));
+    // at most one descriptor per point: a cap of n always holds the result
+    const int rc = pcc_rift_batched(ws, all.data(), n, (int)sizeof(PointT), inten.data(), off.data(), n_clouds, normal_radius, gradient_radius, rift_radius,
+                                    nr_distance_bins, nr_gradient_bins, flat.data(), rows.data(), n, desc_off.data(), PCC_HOST, nullptr);
+    pcc_destroy(ws);
+    check(rc);
+    descriptors.assign((size_t)n_clouds, std::vector<Histogram32>());
+    kept_rows.assign((size_t)n_clouds, std::vector<int>());
+    for (int64_t c = 0; c < n_clouds; ++c) {
+        for (int64_t i = desc_off[c]; i < desc_off[c + 1]; ++i) {
+            Histogram32 h;
+            for (int k = 0; k < 32; ++k) h.histogram[k] = k < nb ? flat[(size_t)i * nb + k] : 0.f;
+            descriptors[c].push_back(h);
+            kept_rows[c].push_back(rows[(size_t)i]);
+        }
+    }
+}
 
 // matchRIFTFeaturesKnn (src/comparator.cpp:560-588): KdTreeFLANN<Histogram<32>> over descriptors1, nearestKSearch(k = 1) for every
 // descriptor of descriptors2, kept when the squared distance is < 0.05.  The returned vector starts with one 0, as the reference's

@@ -109,6 +109,18 @@ int pcc_intensity_gradient(pcc_index *idx, const void *q, int64_t nq, int stride
  * centre and p0; each histogram is normalised to unit Frobenius norm (an all-zero one stays zero). */
 int pcc_rift(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, double radius, const float *gradient4,
              int n_distance_bins, int n_gradient_bins, float *out, int mem, void *stream);
+/* processRIFT (src/comparator.cpp:590-684) on every cluster of a concatenated cloud in one call: per cluster, pcc_normals_radius
+ * (viewpoint 0) -> drop the rows with a non-finite normal -> pcc_intensity_gradient and pcc_rift on the remaining points -> drop the
+ * rows with a non-finite bin, bit for bit as those calls on the cluster alone.  Cluster c is rows [cloud_offsets[c],
+ * cloud_offsets[c+1]) of pts (rows of stride_bytes with x, y, z first); intensity[n] is one float per row (rgbToIntensity).
+ * cloud_offsets (HOST, n_clouds + 1 entries, n_clouds <= 2^24) starts at 0, ends at n and never decreases, empty clusters allowed;
+ * radii finite and >= 0, 1 <= nd*ng <= 32.  out_desc gets the surviving descriptors (nd*ng floats each, PCL's bin order) in
+ * (cluster, row) order and out_rows their cluster-LOCAL row numbers, at most `cap` rows; desc_offsets (HOST, n_clouds + 1) always
+ * gets the full layout, desc_offsets[n_clouds] = total (cap = 0 only counts).  Host round trips do not depend on n_clouds.
+ * `idx` is the workspace: after a call with n > 0 it indexes the concatenated input (cell max(radii)); with n = 0 it is untouched. */
+int pcc_rift_batched(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, const float *intensity, const int64_t *cloud_offsets,
+                     int64_t n_clouds, double normal_radius, double gradient_radius, double rift_radius, int n_distance_bins, int n_gradient_bins,
+                     float *out_desc, int32_t *out_rows, int64_t cap, int64_t *desc_offsets, int mem, void *stream);
 
 /* SIFTKeypoint<PointXYZRGB, PointWithScale> (src/comparator.cpp:449-465: min_scale 0.005, 5 octaves, 5 scales per octave,
  * min_contrast 0.001) [up].  DESIGN.md section 2 records the reading of PCL's sift_keypoint.hpp these restate.

@@ -75,6 +75,9 @@ struct pcc_index {
     // pcc_sift_keypoints_batched: segment label per sorted position of the current grid (segment_labels), the octave's segment
     // offsets, per-segment tables, per-row segment labels of the segmented VoxelGrid and the keypoints staged across octaves
     pcc::Buf seg_label, seg_off, sift_tab, sift_lab, sift_stage;
+    // pcc_rift_batched: one stage's rows derived from the master rows (offsets, keys, scan scratch), the staged intensity, per-row
+    // normals, gradients and descriptors, the survivor scan, the cluster offsets and bounds, and the compacted rows of a PCC_HOST call
+    pcc::Buf rift_off, rift_keys, rift_tmp, rift_in, rift_nrm, rift_grad, rift_desc, rift_pos, rift_tab, rift_out, rift_row;
     uint64_t grid_gen = 0;     // bumped by pcc_build / pcc_adopt
     void *comm = nullptr;      // ncclComm_t handed to pcc_comm_init (not owned); rank / world of this process in it
     int comm_rank = 0, comm_world = 1;
@@ -174,6 +177,12 @@ int segment_labels(pcc_index *idx, const int64_t *d_off, int n_seg, cudaStream_t
 int segmented_sorted_rows(pcc_index *idx, const uint32_t *seg, double radius, const int64_t **d_off, const nkey_t **keys, cudaStream_t s);
 // pcc_sift_dog over segmented_sorted_rows (device pointers, no checks); rows of unindexed points are NaN
 int sift_dog_segmented(pcc_index *idx, const uint32_t *seg, const float *values, const float *scales, int n_scales, float *out, cudaStream_t s);
+// processRIFT's normals, gradient and RIFT stages over one segmented_sorted_rows pass at the largest radius (pcc_rift_batched): each
+// stage's rows are a prefix of the master rows, less the neighbours with a non-finite normal for the gradient and RIFT stages, and
+// empty for a query whose own normal is not finite.  normals / gradient (float4) and desc (nd * ng floats) have one row per input row;
+// rows of unindexed points get NaN normals and undefined gradients and descriptors.  All pointers are device pointers.
+int rift_segmented(pcc_index *idx, const uint32_t *seg, const float *intensity, double normal_radius, double gradient_radius, double rift_radius,
+                   int nd, int ng, float4 *normals, float4 *gradient, float *desc, cudaStream_t s);
 // pcc_first_within restricted to the query's segment: query t belongs to segment segment_of(d_qoff, t), the indexed points carry
 // their segment in seg, and out[t] is relative to that segment's first row (d_poff).  q, d_qoff, d_poff and out are device pointers.
 int first_within_segmented(pcc_index *idx, const uint32_t *seg, const float4 *q, int64_t nq, const int64_t *d_qoff, const int64_t *d_poff, int n_seg,

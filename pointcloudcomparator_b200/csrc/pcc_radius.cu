@@ -586,6 +586,36 @@ __global__ void __launch_bounds__(128) first_within_seg_kernel(Grid g, const uin
     }
     out[t] = best == INT_MAX ? -1 : best - (int32_t)__ldg(poff + sq);
 }
+// processRIFT's rows at radius r from master rows at R >= r: rows are sorted by (d2, index), so the stage's row is the prefix with
+// d2 < r2.  With `normals`, only neighbours whose normal is finite are kept and the row of a query whose own normal is not is empty:
+// the rows of processRIFT's filtered cloud, in the same order, under the original indices.
+template <class F>
+__device__ __forceinline__ void rift_stage_row(const int64_t *__restrict__ moff, const nkey_t *__restrict__ mkeys, int64_t row, float r2,
+                                               const float4 *__restrict__ normals, F &&f) {
+    if (normals) { const float4 m = __ldg(normals + row); if (!finite3(m.x, m.y, m.z)) return; }
+    const int64_t e = moff[row + 1];
+    for (int64_t j = moff[row]; j < e; ++j) {
+        const nkey_t k = mkeys[j];
+        if (!(key_d2(k) < r2)) break;
+        if (normals) { const float4 m = __ldg(normals + (uint32_t)k); if (!finite3(m.x, m.y, m.z)) continue; }
+        f(k);
+    }
+}
+__global__ void rift_stage_count_kernel(const int64_t *__restrict__ moff, const nkey_t *__restrict__ mkeys, int64_t rows, float r2,
+                                        const float4 *__restrict__ normals, int64_t *__restrict__ counts) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t > rows) return;
+    int64_t n = 0;
+    if (t < rows) rift_stage_row(moff, mkeys, t, r2, normals, [&](nkey_t) { ++n; });
+    counts[t] = n;
+}
+__global__ void rift_stage_copy_kernel(const int64_t *__restrict__ moff, const nkey_t *__restrict__ mkeys, int64_t rows, float r2,
+                                       const float4 *__restrict__ normals, const int64_t *__restrict__ offsets, nkey_t *__restrict__ keys) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= rows) return;
+    nkey_t *o = keys + offsets[t];
+    rift_stage_row(moff, mkeys, t, r2, normals, [&](nkey_t k) { *o++ = k; });
+}
 
 // ---- EuclideanClusterExtraction: lock-free union-find over sorted positions ----
 // Loads bypass L1 (__ldcg) so a root that another SM has just hooked is seen in L2; a stale value is still
@@ -875,6 +905,55 @@ int pcc::first_within_segmented(pcc_index *idx, const uint32_t *seg, const float
     if (nq == 0) return PCC_OK;
     const float r2_cover = (float)(thr * thr * (1.0 + 1e-5));       // as pcc_first_within
     first_within_seg_kernel<<<nblocks(nq, 128), 128, 0, s>>>(idx->grid(), seg, q, nq, d_qoff, d_poff, n_seg, thr, r2_cover, ring0(idx, thr), out);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    return PCC_OK;
+}
+// one stage's rows (rift_stage_row) into idx->rift_off / idx->rift_keys: count, scan, copy.  Every stage row set is a subset of the
+// master rows, whose keys fit in idx->keys64, so rift_keys is sized from that buffer and no total is read back.
+static int rift_stage_rows(pcc_index *idx, const int64_t *moff, const nkey_t *mkeys, double radius, const float4 *normals, const int64_t **off_out,
+                           const nkey_t **keys_out, cudaStream_t s) {
+    const int64_t rows = idx->n_input;
+    const float r2 = (float)(radius * radius);
+    PCC_TRY(idx->rift_off.reserve((size_t)(rows + 1) * 8));
+    PCC_TRY(idx->rift_keys.reserve(idx->keys64.cap));
+    int64_t *off = idx->rift_off.as<int64_t>();
+    nkey_t *keys = idx->rift_keys.as<nkey_t>();
+    rift_stage_count_kernel<<<nblocks(rows + 1, 128), 128, 0, s>>>(moff, mkeys, rows, r2, normals, off);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    size_t tmp = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp, off, off, (int)(rows + 1), s);
+    PCC_TRY(idx->rift_tmp.reserve(tmp));
+    PCC_CUDA(cub::DeviceScan::ExclusiveSum(idx->rift_tmp.p, tmp, off, off, (int)(rows + 1), s));
+    g_launches += 2;
+    rift_stage_copy_kernel<<<nblocks(rows, 128), 128, 0, s>>>(moff, mkeys, rows, r2, normals, off, keys);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    *off_out = off; *keys_out = keys;
+    return PCC_OK;
+}
+int pcc::rift_segmented(pcc_index *idx, const uint32_t *seg, const float *intensity, double normal_radius, double gradient_radius, double rift_radius,
+                        int nd, int ng, float4 *normals, float4 *gradient, float *desc, cudaStream_t s) {
+    const int64_t *moff = nullptr; const nkey_t *mkeys = nullptr;
+    PCC_TRY(segmented_sorted_rows(idx, seg, std::max(normal_radius, std::max(gradient_radius, rift_radius)), &moff, &mkeys, s));
+    if (!idx->inv_valid) PCC_TRY(rebuild_inverse(idx, s));
+    if (!idx->all_rows_indexed) PCC_CUDA(cudaMemsetAsync(normals, 0xFF, (size_t)idx->n_input * 16, s));     // unindexed rows: NaN normals, dropped
+    if (idx->n_indexed == 0) return PCC_OK;
+    const QueryView v{nullptr, nullptr, idx->n_indexed, true};
+    const uint32_t *inv = idx->inv_pos.as<uint32_t>();
+    const unsigned nbk = nblocks(idx->n_indexed, 128);
+    const int64_t *off = nullptr; const nkey_t *keys = nullptr;
+    PCC_TRY(rift_stage_rows(idx, moff, mkeys, normal_radius, nullptr, &off, &keys, s));
+    normals_rows_kernel<<<nbk, 128, 0, s>>>(idx->grid(), v, off, keys, inv, 0.f, 0.f, 0.f, normals);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    PCC_TRY(rift_stage_rows(idx, moff, mkeys, gradient_radius, normals, &off, &keys, s));
+    gradient_rows_kernel<<<nbk, 128, 0, s>>>(idx->grid(), v, off, keys, inv, intensity, normals, gradient);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    PCC_TRY(rift_stage_rows(idx, moff, mkeys, rift_radius, normals, &off, &keys, s));
+    rift_rows_kernel<<<nbk, 128, 0, s>>>(idx->grid(), v, off, keys, inv, gradient, (float)rift_radius, nd, ng, desc);
     PCC_LAUNCHED();
     PCC_CUDA(cudaGetLastError());
     return PCC_OK;

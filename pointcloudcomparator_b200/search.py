@@ -434,6 +434,45 @@ def process_rift(xyz, rgb, normal_radius: float = 0.03, gradient_radius: float =
     return desc[keep2], keep1[keep2].astype(np.int64)
 
 
+def process_rift_batched(xyz, rgb, offsets, normal_radius: float = 0.03, gradient_radius: float = 0.03, rift_radius: float = 0.05,
+                         nr_distance_bins: int = 4, nr_gradient_bins: int = 8, device: int = 0):
+    """process_rift on every cluster [offsets[c], offsets[c+1]) of xyz / rgb in one pcc_rift_batched call: returns (descriptors [m, nd*ng],
+    desc_offsets int64 [n_clouds + 1], kept_rows int64 [m]); rows desc_offsets[c]:desc_offsets[c+1] are process_rift of cluster c, bit for
+    bit, with cluster-LOCAL kept rows.  numpy inputs go through PCC_HOST; a CUDA tensor xyz keeps the call and its outputs on the device,
+    on the current stream."""
+    off = np.ascontiguousarray(np.asarray(offsets), np.int64)
+    n_clouds = off.shape[0] - 1
+    desc_off = np.zeros(max(n_clouds, 0) + 1, np.int64)
+    nb = int(nr_distance_bins) * int(nr_gradient_bins)
+    inten = rgb_to_intensity(rgb)
+    if _is_cuda(xyz):
+        ptr, n, stride, mem, keep = _rows(xyz)
+        it = torch.as_tensor(inten, device=xyz.device)
+        ip = it.data_ptr()
+        alloc = lambda shape, dt: torch.empty(shape, dtype=dt, device=xyz.device)      # noqa: E731
+        f32, i32 = torch.float32, torch.int32
+    else:
+        ptr, n, stride, mem, keep = _rows(np.asarray(xyz, np.float32))
+        ip = inten.ctypes.data
+        alloc = lambda shape, dt: np.empty(shape, dt)                                   # noqa: E731
+        f32, i32 = np.float32, np.int32
+    L = _lib.lib()
+    ws = GridSearch(device)
+    cap = max(n, 1)
+    while True:
+        out = alloc((cap, max(nb, 1)), f32)
+        rows = alloc((cap,), i32)
+        op, rp = (out.data_ptr(), rows.data_ptr()) if mem == DEVICE else (out.ctypes.data, rows.ctypes.data)
+        check(L.pcc_rift_batched(ws._h, ptr, n, stride, ip, off.ctypes.data, n_clouds, float(normal_radius), float(gradient_radius), float(rift_radius),
+                                 int(nr_distance_bins), int(nr_gradient_bins), op, rp, cap, desc_off.ctypes.data, mem, _stream(ws.device)))
+        total = int(desc_off[-1])
+        if total <= cap:
+            break
+        cap = total
+    kept = rows[:total].to(torch.int64) if mem == DEVICE else rows[:total].astype(np.int64)
+    return out[:total], desc_off, kept
+
+
 def sift_field_values(rgb):
     """PCL 1.7 SIFTKeypointFieldSelector<PointXYZRGB>: float(299 r + 587 g + 114 b) / 1000.0f (integer sum, one fp32 division).
     Not the XYZRGB -> XYZI weights of rgb_to_intensity.  rgb[n, 3] uint8 (r, g, b) -> float32[n]."""
