@@ -19,6 +19,8 @@
 //   pcc::IntensityGradientEstimation <- pcl::IntensityGradientEstimation (src/comparator.cpp:649-656)
 //   pcc::RIFTEstimation              <- pcl::RIFTEstimation              (src/comparator.cpp:659-673)
 //   pcc::processRIFTBatched          <- processRIFT on every cluster     (src/comparator.cpp:590-684, 1224-1366)
+//   pcc::findPointNeighboursBatched, pcc::RegionGrowingRGBBatched
+//                                    <- color_growing_segmentation on every cluster (src/segmentation.cpp:161-216, src/comparator.cpp:1457-1460)
 // There is no CPU fallback: a failing CUDA call throws pcc::Error.
 #ifndef PCC_GRID_SEARCH_HPP_
 #define PCC_GRID_SEARCH_HPP_
@@ -449,12 +451,12 @@ class RegionGrowingRGB {
         tree_->setKHint(table_k_);
         if (tree_->getInputCloud() != input_) tree_->setInputCloud(input_);
         std::vector<int> nbrs; std::vector<float> d2;
-        const int k = findPointNeighbours(*tree_, table_k_, nbrs, d2);
+        findPointNeighbours(*tree_, table_k_, nbrs, d2);          // rows of stride table_k_; a cluster under table_k_ points ends its rows with -1
         labels_.assign(n, -1);
         int64_t nc = 0;
         const uint32_t *rgba = reinterpret_cast<const uint32_t *>(reinterpret_cast<const char *>(input_->points.data()) + rgba_off_);
-        check(pcc_region_growing_rgb(nbrs.data(), d2.data(), (int64_t)n, k, rgba, (int)sizeof(PointT), distance_, point_color_, region_color_,
-                                     std::min(grow_k_, k), min_size_, max_size_, labels_.data(), &nc));
+        check(pcc_region_growing_rgb(nbrs.data(), d2.data(), (int64_t)n, table_k_, rgba, (int)sizeof(PointT), distance_, point_color_, region_color_,
+                                     std::min(grow_k_, table_k_), min_size_, max_size_, labels_.data(), &nc));
         clusters.resize((size_t)nc);
         for (size_t i = 0; i < n; ++i) if (labels_[i] >= 0) clusters[(size_t)labels_[i]].indices.push_back((int)i);
     }
@@ -463,6 +465,85 @@ class RegionGrowingRGB {
     typename search::GridSearch<PointT>::Ptr tree_;
     typename search::GridSearch<PointT>::PointCloudConstPtr input_;
     std::vector<int32_t> labels_;
+    int rgba_off_, table_k_ = 100, grow_k_ = 30;
+    int64_t min_size_ = 1, max_size_ = std::numeric_limits<int>::max();
+    float distance_ = 10.f, point_color_ = 1225.f, region_color_ = 10.f;          // PCL 1.7 constructor defaults
+};
+
+// findPointNeighbours of every cluster in one call (pcc_knn_batched): neighbours[c] / sqr_distances[c] get exactly the table
+// findPointNeighbours fills for cluster c alone (stride k, cluster-local indices, -1 / +inf past the cluster's k_eff); returns k_eff per
+// cluster.  Clusters are copied into one concatenated cloud for the call.
+template <typename PointT>
+inline std::vector<int> findPointNeighboursBatched(const std::vector<typename search::GridSearch<PointT>::PointCloudConstPtr> &clusters, int k,
+                                                   std::vector<std::vector<int> > &neighbours, std::vector<std::vector<float> > &sqr_distances, int device = 0) {
+    std::vector<PointT> all;
+    std::vector<int64_t> off(1, 0);
+    for (const auto &c : clusters) {
+        if (!c) throw Error("findPointNeighboursBatched: null input cloud");
+        all.insert(all.end(), c->points.begin(), c->points.end());
+        off.push_back((int64_t)all.size());
+    }
+    const int64_t n_clouds = (int64_t)clusters.size(), n = (int64_t)all.size();
+    std::vector<int> fi((size_t)n * (size_t)std::max(k, 0)), keff((size_t)n_clouds + 1);
+    std::vector<float> fd(fi.size());
+    pcc_index *ws = nullptr;
+    check(pcc_create(device, &ws));
+    const int rc = pcc_knn_batched(ws, all.data(), n, (int)sizeof(PointT), off.data(), n_clouds, k, fi.data(), fd.data(), keff.data(), PCC_HOST, nullptr);
+    pcc_destroy(ws);
+    check(rc);
+    neighbours.assign((size_t)n_clouds, std::vector<int>());
+    sqr_distances.assign((size_t)n_clouds, std::vector<float>());
+    for (int64_t c = 0; c < n_clouds; ++c) {
+        neighbours[c].assign(fi.begin() + off[c] * k, fi.begin() + off[c + 1] * k);
+        sqr_distances[c].assign(fd.begin() + off[c] * k, fd.begin() + off[c + 1] * k);
+    }
+    keff.resize((size_t)n_clouds);
+    return keff;
+}
+
+// RegionGrowingRGB over every cluster of a cloud in one call (pcc_region_growing_rgb_batched), as computeSimilarity runs
+// color_growing_segmentation on both clouds of every matched pair (src/comparator.cpp:1457-1460): extract fills clusters[c] with exactly what
+// RegionGrowingRGB::extract returns on cluster c alone, members as cluster-local rows.  One GPU pass builds every cluster's table; the grow /
+// merge runs on the host, one cluster after another.  The reference segments only clouds of more than 10 points
+// (src/segmentation.cpp:167): that test stays with the caller.  Setters and defaults are RegionGrowingRGB's.
+template <typename PointT>
+class RegionGrowingRGBBatched {
+  public:
+    explicit RegionGrowingRGBBatched(int rgba_offset = 16, int device = 0) : rgba_off_(rgba_offset) { check(pcc_create(device, &ws_)); }
+    ~RegionGrowingRGBBatched() { pcc_destroy(ws_); }
+    RegionGrowingRGBBatched(const RegionGrowingRGBBatched &) = delete;
+    RegionGrowingRGBBatched &operator=(const RegionGrowingRGBBatched &) = delete;
+    void setInputClouds(const std::vector<typename search::GridSearch<PointT>::PointCloudConstPtr> &clouds) { inputs_ = clouds; }
+    void setDistanceThreshold(float d) { distance_ = d; }
+    void setPointColorThreshold(float t) { point_color_ = t; }
+    void setRegionColorThreshold(float t) { region_color_ = t; }
+    void setNumberOfRegionNeighbours(unsigned int k) { table_k_ = (int)k; }
+    void setNumberOfNeighbours(unsigned int k) { grow_k_ = (int)k; }
+    void setMinClusterSize(int n) { min_size_ = n; }
+    void setMaxClusterSize(int n) { max_size_ = n; }
+    void extract(std::vector<std::vector<PointIndices> > &clusters) {
+        std::vector<PointT> all;
+        std::vector<int64_t> off(1, 0);
+        for (const auto &c : inputs_) {
+            if (!c) throw Error("RegionGrowingRGBBatched: null input cloud");
+            all.insert(all.end(), c->points.begin(), c->points.end());
+            off.push_back((int64_t)all.size());
+        }
+        const int64_t n_clouds = (int64_t)inputs_.size();
+        std::vector<int32_t> labels(all.size());
+        std::vector<int64_t> nc((size_t)n_clouds + 1);
+        check(pcc_region_growing_rgb_batched(ws_, all.data(), (int64_t)all.size(), (int)sizeof(PointT), rgba_off_, off.data(), n_clouds, table_k_, distance_,
+                                             point_color_, region_color_, std::min(grow_k_, table_k_), min_size_, max_size_, labels.data(), nc.data(),
+                                             PCC_HOST, nullptr));
+        clusters.assign((size_t)n_clouds, std::vector<PointIndices>());
+        for (int64_t c = 0; c < n_clouds; ++c) {
+            clusters[c].resize((size_t)nc[c]);
+            for (int64_t i = off[c]; i < off[c + 1]; ++i) if (labels[i] >= 0) clusters[c][(size_t)labels[i]].indices.push_back((int)(i - off[c]));
+        }
+    }
+  private:
+    pcc_index *ws_ = nullptr;
+    std::vector<typename search::GridSearch<PointT>::PointCloudConstPtr> inputs_;
     int rgba_off_, table_k_ = 100, grow_k_ = 30;
     int64_t min_size_ = 1, max_size_ = std::numeric_limits<int>::max();
     float distance_ = 10.f, point_color_ = 1225.f, region_color_ = 10.f;          // PCL 1.7 constructor defaults

@@ -67,6 +67,15 @@ int pcc_grid_info(const pcc_index *idx, double out[5]);
  * Rows have stride k; entries past *k_eff = min(k, pcc_size) and rows of non-finite queries hold (-1, +inf). */
 int pcc_knn(pcc_index *idx, const void *q, int64_t nq, int stride_bytes, int k, int32_t *out_idx, float *out_d2,
             int *k_eff, int mem, void *stream);
+/* RegionGrowingRGB::findPointNeighbours (src/segmentation.cpp:190) on every cluster of a concatenated cloud in one call.  Cluster c is
+ * rows [cloud_offsets[c], cloud_offsets[c+1]) of pts; cloud_offsets (HOST, n_clouds + 1 entries, n_clouds <= 2^24) starts at 0, ends at
+ * n and never decreases, empty clusters allowed; 1 <= k <= PCC_MAX_K.  Row i of out_idx / out_d2 (stride k, input order) is, bit for
+ * bit, row i - cloud_offsets[c] of pcc_knn(q == NULL, k) on cluster c alone: cluster-LOCAL indices, (d2, index) order, entries past
+ * min(k, finite points of c) and rows of non-finite points (-1, +inf).  k_eff (HOST, n_clouds) gets min(k, finite points) per cluster.
+ * Host round trips do not depend on n_clouds.  `idx` is the workspace: after a call with n > 0 it indexes the concatenated input
+ * (k_hint = k); with n = 0 it is untouched. */
+int pcc_knn_batched(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, const int64_t *cloud_offsets, int64_t n_clouds, int k,
+                    int32_t *out_idx, float *out_d2, int32_t *k_eff, int mem, void *stream);
 
 /* Search::radiusSearch, batched overload (src/segmentation.cpp:126,131 r=0.05; src/comparator.cpp:631,655,666 r=0.03/0.05).
  * KdTreeFLANN::radiusSearch [up]: d2 < float(radius*radius) strictly; max_nn = 0 means unlimited, else the max_nn
@@ -226,6 +235,15 @@ int pcc_region_growing(const int32_t *neighbours, int64_t n, int k, const float 
 int pcc_region_growing_rgb(const int32_t *neighbours, const float *sqr_distances, int64_t n, int k, const uint32_t *rgba, int rgba_stride_bytes,
                            float distance_threshold, float point_color_threshold, float region_color_threshold, int grow_neighbours,
                            int64_t min_size, int64_t max_size, int32_t *labels, int64_t *n_clusters);
+/* color_growing_segmentation on every cluster of a concatenated cloud in one call: pcc_knn_batched, then pcc_region_growing_rgb on each
+ * cluster's slice of the table (stride k, cluster-LOCAL indices), one cluster after another on the host.  pts and cloud_offsets as
+ * pcc_knn_batched; the packed 0x00RRGGBB colour word sits at rgb_offset_bytes of every row (pcl::PointXYZRGB: stride 32, offset 16).
+ * labels (HOST, n) gets each point's cluster-LOCAL label in PCL's order, or -1; n_clusters (HOST, n_clouds) each cluster's count -- for
+ * every cluster what pcc_knn(q == NULL, k) + pcc_region_growing_rgb give on that cluster alone.  The reference only segments a cloud of
+ * more than 10 points (src/segmentation.cpp:167); that test stays with the caller.  `idx` as pcc_knn_batched. */
+int pcc_region_growing_rgb_batched(pcc_index *idx, const void *pts, int64_t n, int stride_bytes, int rgb_offset_bytes, const int64_t *cloud_offsets,
+                                   int64_t n_clouds, int k, float distance_threshold, float point_color_threshold, float region_color_threshold,
+                                   int grow_neighbours, int64_t min_size, int64_t max_size, int32_t *labels, int64_t *n_clusters, int mem, void *stream);
 
 /* matchRIFTFeaturesKnn (src/comparator.cpp:560-588): KdTreeFLANN<Histogram<32>> over `ref`, nearestKSearch(k = 1) for every row
  * of `qry` [up].  Exact brute force in descriptor space: d2 accumulated sequentially over the first `dim` floats of a row (fp32, no

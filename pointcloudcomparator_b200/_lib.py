@@ -22,7 +22,7 @@ SYMBOLS = [
     "pcc_knn", "pcc_radius_count", "pcc_radius_fill", "pcc_knn_mean_dist", "pcc_sor_threshold", "pcc_normals_knn",
     "pcc_normals_radius", "pcc_icp_step", "pcc_icp_align", "pcc_umeyama_from_sums", "pcc_euclidean_labels", "pcc_first_within",
     "pcc_export", "pcc_adopt", "pcc_set_timing", "pcc_last_kernel_ms", "pcc_ece_init", "pcc_ece_link_range", "pcc_ece_absorb", "pcc_ece_finish", "pcc_voxel_grid", "pcc_descriptor_nn", "pcc_region_growing",
-    "pcc_region_growing_rgb", "pcc_intensity_gradient", "pcc_rift", "pcc_sift_dog", "pcc_sift_extrema", "pcc_sift_keypoints", "pcc_sift_keypoints_batched", "pcc_rift_batched", "pcc_comm_init", "pcc_comm_info", "pcc_broadcast_index", "pcc_gather", "pcc_allreduce_f64",
+    "pcc_region_growing_rgb", "pcc_intensity_gradient", "pcc_rift", "pcc_sift_dog", "pcc_sift_extrema", "pcc_sift_keypoints", "pcc_sift_keypoints_batched", "pcc_rift_batched", "pcc_knn_batched", "pcc_region_growing_rgb_batched", "pcc_comm_init", "pcc_comm_info", "pcc_broadcast_index", "pcc_gather", "pcc_allreduce_f64",
 ]
 
 
@@ -62,6 +62,8 @@ def lib():
     L.pcc_sift_keypoints.argtypes = [vp, vp, i64, i32, i32, C.c_float, i32, i32, C.c_float, vp, i64, C.POINTER(i64), i32, vp]
     L.pcc_sift_keypoints_batched.argtypes = [vp, vp, i64, i32, i32, vp, i64, C.c_float, i32, i32, C.c_float, dbl, vp, vp, i64, vp, i32, vp]
     L.pcc_rift_batched.argtypes = [vp, vp, i64, i32, vp, vp, i64, dbl, dbl, dbl, i32, i32, vp, vp, i64, vp, i32, vp]
+    L.pcc_knn_batched.argtypes = [vp, vp, i64, i32, vp, i64, i32, vp, vp, vp, i32, vp]
+    L.pcc_region_growing_rgb_batched.argtypes = [vp, vp, i64, i32, i32, vp, i64, i32, C.c_float, C.c_float, C.c_float, i32, i64, i64, vp, vp, i32, vp]
     L.pcc_icp_step.argtypes = [vp, vp, i64, i32, C.POINTER(C.c_float), C.POINTER(dbl), C.POINTER(i64), vp, vp, i32, vp]
     L.pcc_icp_align.argtypes = [vp, vp, i64, i32, i32, C.POINTER(C.c_float), C.POINTER(i32), C.POINTER(dbl), C.POINTER(i32), i32, vp]
     L.pcc_umeyama_from_sums.argtypes = [C.POINTER(dbl), i64, C.POINTER(C.c_float)]

@@ -335,7 +335,7 @@ void pcc_destroy(pcc_index *idx) {
                    &idx->sift_cloud[0], &idx->sift_cloud[1], &idx->sift_val, &idx->sift_dog, &idx->sift_in, &idx->sift_nbr, &idx->sift_d2, &idx->sift_flag, &idx->sift_pos,
                    &idx->sift_row, &idx->sift_col, &idx->sift_kp, &idx->seg_label, &idx->seg_off, &idx->sift_tab, &idx->sift_lab, &idx->sift_stage,
                    &idx->rift_off, &idx->rift_keys, &idx->rift_tmp, &idx->rift_in, &idx->rift_nrm, &idx->rift_grad, &idx->rift_desc, &idx->rift_pos,
-                   &idx->rift_tab, &idx->rift_out, &idx->rift_row};
+                   &idx->rift_tab, &idx->rift_out, &idx->rift_row, &idx->knnb_tab};
     for (Buf *b : bufs) b->release();
     if (idx->h_pinned) cudaFreeHost(idx->h_pinned);
     if (idx->aux_stream) cudaStreamDestroy(idx->aux_stream);

@@ -78,6 +78,8 @@ struct pcc_index {
     // pcc_rift_batched: one stage's rows derived from the master rows (offsets, keys, scan scratch), the staged intensity, per-row
     // normals, gradients and descriptors, the survivor scan, the cluster offsets and bounds, and the compacted rows of a PCC_HOST call
     pcc::Buf rift_off, rift_keys, rift_tmp, rift_in, rift_nrm, rift_grad, rift_desc, rift_pos, rift_tab, rift_out, rift_row;
+    // pcc_knn_batched: the cluster offsets and the finite points per cluster
+    pcc::Buf knnb_tab;
     uint64_t grid_gen = 0;     // bumped by pcc_build / pcc_adopt
     void *comm = nullptr;      // ncclComm_t handed to pcc_comm_init (not owned); rank / world of this process in it
     int comm_rank = 0, comm_world = 1;
@@ -175,6 +177,10 @@ int segment_labels(pcc_index *idx, const int64_t *d_off, int n_seg, cudaStream_t
 // the indexed cloud's own radius rows with neighbours of the query's segment only, sorted by (d2, index): offsets (n_input + 1,
 // in idx->out_l) and keys (idx->keys64); rows of unindexed points are empty
 int segmented_sorted_rows(pcc_index *idx, const uint32_t *seg, double radius, const int64_t **d_off, const nkey_t **keys, cudaStream_t s);
+// pcc_knn(q == NULL, k) of every segment alone, for any 1 <= k <= PCC_MAX_K, over the selection path: the dense [n_input, k] table
+// oi / od with segment-LOCAL indices (row - seg_off[segment]), (d2, index) order, rows past min(k, seg_n[segment]) and rows of
+// unindexed points (-1, +inf).  seg_n (finite points per segment), seg_off (n_seg + 1), oi and od are device pointers.
+int knn_select_segmented(pcc_index *idx, const uint32_t *seg, const uint32_t *seg_n, const int64_t *seg_off, int k, int32_t *oi, float *od, cudaStream_t s);
 // pcc_sift_dog over segmented_sorted_rows (device pointers, no checks); rows of unindexed points are NaN
 int sift_dog_segmented(pcc_index *idx, const uint32_t *seg, const float *values, const float *scales, int n_scales, float *out, cudaStream_t s);
 // processRIFT's normals, gradient and RIFT stages over one segmented_sorted_rows pass at the largest radius (pcc_rift_batched): each

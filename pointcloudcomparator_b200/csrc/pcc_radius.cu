@@ -255,6 +255,96 @@ __global__ void __launch_bounds__(128) select_fill_kernel(Grid g, QueryView v, c
     });
     if (n & 3) { o[0] = make_ulonglong2(p0, p1); o[1] = make_ulonglong2(p2, p3); }
 }
+// select_bound_kernel / select_fill_kernel for the indexed cloud's own rows, admitting a neighbour when its segment is the query's
+// (pcc_knn_batched).  seg_n[s] = finite points of segment s.  Every point outside the block, of any segment, has d2 >= covered_d2(R),
+// so the bracket argument is unchanged.  A query whose block already holds every point of its segment stops growing and brackets
+// by the largest of their distances: a 50-point cluster never walks a union grid it shares with clusters a kilometre away.
+__global__ void __launch_bounds__(128, PCC_SELB) seg_select_bound_kernel(Grid g, const uint32_t *__restrict__ seg, const uint32_t *__restrict__ seg_n, int k,
+                                                                         int64_t *__restrict__ counts, SelParam *__restrict__ params) {
+    __shared__ uint32_t hist_all[kSelBuckets * 128];
+    uint32_t *hist = hist_all + threadIdx.x;
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= g.n) return;
+    const float4 q = __ldg(g.pts + t);
+    const uint32_t sq = __ldg(seg + t), total = __ldg(seg_n + sq);
+    const unsigned kk = min((unsigned)k, total);          // the row holds min(k, points of the segment)
+    const QueryCell c = locate(g, q.x, q.y, q.z);
+    int R = 1, B = -1;
+    unsigned m = 0;
+    float scale = 0.f;
+    auto pick = [&]() {                                    // first bucket whose cumulative count reaches kk
+        unsigned seen = 0;
+        for (int b = 0; b < kSelBuckets; ++b) { seen += hist[b * 128]; if (seen >= kk) { B = b; m = seen; break; } }
+    };
+    for (;;) {
+        const float cov = covered_d2(g, c, R);
+        const bool bounded = cov > 0.f && cov < CUDART_INF_F;
+        unsigned cnt = 0;
+        float mx = 0.f;
+        if (bounded) {
+            scale = (float)kSelBuckets / cov;
+#pragma unroll 8
+            for (int b = 0; b < kSelBuckets; ++b) hist[b * 128] = 0u;
+        }
+        scan_shell(g, c, -1, R, [&](uint32_t pos, float4 p) {
+            if (__ldg(seg + pos) != sq) return;
+            const float d2 = dist2(q.x, q.y, q.z, p.x, p.y, p.z);
+            ++cnt; mx = fmaxf(mx, d2);
+            const float fb = __fmul_rn(d2, scale);
+            if (bounded && fb < (float)kSelBuckets) hist[(int)fb * 128] += 1u;
+        });
+        if (bounded) { pick(); if (B >= 0) break; }
+        if (cnt >= total || cov == CUDART_INF_F) {         // the block holds the whole segment: bracket by its largest distance
+            float hi = fmaxf(mx * 1.0001f, 1e-30f);
+            if (!(hi < CUDART_INF_F)) hi = 3.0e38f;
+            scale = (float)kSelBuckets / hi;
+            if (cnt <= (unsigned)k) { B = kSelBuckets - 1; m = cnt; break; }      // at most k points: all of them
+#pragma unroll 8
+            for (int b = 0; b < kSelBuckets; ++b) hist[b * 128] = 0u;
+            scan_shell(g, c, -1, R, [&](uint32_t pos, float4 p) {
+                if (__ldg(seg + pos) != sq) return;
+                const float fb = __fmul_rn(dist2(q.x, q.y, q.z, p.x, p.y, p.z), scale);
+                if (fb < (float)kSelBuckets) hist[(int)fb * 128] += 1u;
+            });
+            pick();                                        // every one of the cnt > k points is in a bucket: B is found
+            break;
+        }
+        R = cnt > 0 ? R + 1 : next_ring(g, R, CUDART_INF_F);
+    }
+    counts[__float_as_int(q.w)] = (m + 3u) & ~3u;
+    SelParam sp; sp.scale = scale; sp.bucket = B; sp.R = R; sp.pad = 0;
+    params[__float_as_int(q.w)] = sp;
+}
+// keys carry segment-LOCAL indices (row - seg_off[segment]): within one segment they order as the global ones do
+__global__ void __launch_bounds__(128) seg_select_fill_kernel(Grid g, const uint32_t *__restrict__ seg, const int64_t *__restrict__ seg_off,
+                                                              const int64_t *__restrict__ offsets, const SelParam *__restrict__ params, nkey_t *__restrict__ keys) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= g.n) return;
+    const float4 q = __ldg(g.pts + t);
+    const int64_t row = __float_as_int(q.w);
+    if (offsets[row + 1] == offsets[row]) return;
+    const uint32_t sq = __ldg(seg + t), base = (uint32_t)__ldg(seg_off + sq);
+    const SelParam sp = params[row];
+    const QueryCell c = locate(g, q.x, q.y, q.z);
+    ulonglong2 *o = reinterpret_cast<ulonglong2 *>(keys + offsets[row]);
+    const float edge = (float)(sp.bucket + 1) / sp.scale;
+    const float limit = (float)(sp.bucket + 1);
+    nkey_t p0 = PCC_EMPTY_KEY, p1 = PCC_EMPTY_KEY, p2 = PCC_EMPTY_KEY, p3 = PCC_EMPTY_KEY;
+    int n = 0;
+    scan_clipped(g, c, -1, sp.R, to_cell_units(g, edge * 1.00001f), [&](uint32_t pos, float4 p) {
+        if (__ldg(seg + pos) != sq) return;
+        const float d2 = dist2(q.x, q.y, q.z, p.x, p.y, p.z);
+        const float fb = __fmul_rn(d2, sp.scale);
+        if (fb < (float)kSelBuckets && (float)(int)fb < limit) {
+            const nkey_t key = make_key(d2, __float_as_uint(p.w) - base);
+            const int slot = n & 3;
+            if (slot == 0) p0 = key; else if (slot == 1) p1 = key; else if (slot == 2) p2 = key; else p3 = key;
+            ++n;
+            if (slot == 3) { o[0] = make_ulonglong2(p0, p1); o[1] = make_ulonglong2(p2, p3); o += 2; p0 = p1 = p2 = p3 = PCC_EMPTY_KEY; }
+        }
+    });
+    if (n & 3) { o[0] = make_ulonglong2(p0, p1); o[1] = make_ulonglong2(p2, p3); }
+}
 // first k keys of every row -> the dense [rows, k] result, (-1, +inf) padded
 __global__ void select_unpack_kernel(const int64_t *__restrict__ offsets, const nkey_t *__restrict__ keys, int64_t rows, int k, int32_t *__restrict__ idx, float *__restrict__ d2) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -809,6 +899,25 @@ int knn_select_rows(pcc_index *idx, const Queries &qs, int k, int64_t *d_offsets
     PCC_CUDA(cudaGetLastError());
     return sort_rows ? sort_csr_rows(idx, qs.rows, d_offsets, total, keys, s) : PCC_OK;
 }
+// the first k keys of every unsorted selection row -> the dense [rows, k] result (device pointers)
+static int select_unpack_rows(pcc_index *idx, int64_t rows, int k, int64_t *d_off, nkey_t *keys, int64_t total, int32_t *oi, float *od, cudaStream_t s) {
+    PCC_TRY(idx->misc.reserve(256));
+    unsigned *n_long = idx->misc.as<unsigned>();
+    PCC_CUDA(cudaMemsetAsync(n_long, 0, 4, s));
+    select_sort_unpack_kernel<<<nblocks(rows, 4), 128, 0, s>>>(d_off, keys, rows, k, oi, od, n_long);
+    PCC_LAUNCHED();
+    PCC_CUDA(cudaGetLastError());
+    unsigned *h = (unsigned *)idx->h_pinned;
+    PCC_CUDA(cudaMemcpyAsync(h, n_long, 4, cudaMemcpyDeviceToHost, s));
+    PCC_CUDA(cudaStreamSynchronize(s));
+    if (h[0] > 0) {         // rows above 256 keys (large k, or many points tied inside the bracketing bucket): generic row sort, then unpack everything
+        PCC_TRY(sort_csr_rows(idx, rows, d_off, total, keys, s));
+        select_unpack_kernel<<<nblocks(rows * (int64_t)k, 256), 256, 0, s>>>(d_off, keys, rows, k, oi, od);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    return PCC_OK;
+}
 // pcc_knn for k > 32
 int knn_select(pcc_index *idx, const Queries &qs, int k, int32_t *oi, float *od, cudaStream_t s) {
     PCC_TRY(idx->out_l.reserve((size_t)(qs.rows + 1) * 8));
@@ -816,22 +925,7 @@ int knn_select(pcc_index *idx, const Queries &qs, int k, int32_t *oi, float *od,
     nkey_t *keys = nullptr; int64_t total = 0;
     PCC_TRY(knn_select_rows(idx, qs, k, d_off, &keys, &total, false, s));
     if (qs.rows == 0) return PCC_OK;
-    PCC_TRY(idx->misc.reserve(256));
-    unsigned *n_long = idx->misc.as<unsigned>();
-    PCC_CUDA(cudaMemsetAsync(n_long, 0, 4, s));
-    select_sort_unpack_kernel<<<nblocks(qs.rows, 4), 128, 0, s>>>(d_off, keys, qs.rows, k, oi, od, n_long);
-    PCC_LAUNCHED();
-    PCC_CUDA(cudaGetLastError());
-    unsigned *h = (unsigned *)idx->h_pinned;
-    PCC_CUDA(cudaMemcpyAsync(h, n_long, 4, cudaMemcpyDeviceToHost, s));
-    PCC_CUDA(cudaStreamSynchronize(s));
-    if (h[0] > 0) {         // rows above 256 keys (large k, or many points tied inside the bracketing bucket): generic row sort, then unpack everything
-        PCC_TRY(sort_csr_rows(idx, qs.rows, d_off, total, keys, s));
-        select_unpack_kernel<<<nblocks(qs.rows * (int64_t)k, 256), 256, 0, s>>>(d_off, keys, qs.rows, k, oi, od);
-        PCC_LAUNCHED();
-        PCC_CUDA(cudaGetLastError());
-    }
-    return PCC_OK;
+    return select_unpack_rows(idx, qs.rows, k, d_off, keys, total, oi, od, s);
 }
 
 }  // namespace pcc
@@ -886,6 +980,36 @@ int pcc::segmented_sorted_rows(pcc_index *idx, const uint32_t *seg, double radiu
     PCC_LAUNCHED();
     PCC_CUDA(cudaGetLastError());
     return sort_csr_rows(idx, rows, d_off, total, keys, s);
+}
+int pcc::knn_select_segmented(pcc_index *idx, const uint32_t *seg, const uint32_t *seg_n, const int64_t *seg_off, int k, int32_t *oi, float *od, cudaStream_t s) {
+    const int64_t rows = idx->n_input, n = idx->n_indexed;
+    PCC_TRY(idx->out_l.reserve((size_t)(rows + 1) * 8));
+    PCC_TRY(idx->sel_params.reserve((size_t)std::max<int64_t>(rows, 1) * sizeof(SelParam)));
+    int64_t *d_off = idx->out_l.as<int64_t>();
+    SelParam *params = idx->sel_params.as<SelParam>();
+    PCC_CUDA(cudaMemsetAsync(d_off, 0, (size_t)(rows + 1) * sizeof(int64_t), s));
+    if (n > 0) {
+        seg_select_bound_kernel<<<nblocks(n, 128), 128, 0, s>>>(idx->grid(), seg, seg_n, k, d_off, params);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    size_t tmp = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp, d_off, d_off, (int)(rows + 1), s);
+    PCC_TRY(idx->cub_tmp.reserve(tmp));
+    PCC_CUDA(cub::DeviceScan::ExclusiveSum(idx->cub_tmp.p, tmp, d_off, d_off, (int)(rows + 1), s));
+    g_launches += 2;
+    int64_t *h = (int64_t *)idx->h_pinned;
+    PCC_CUDA(cudaMemcpyAsync(h, d_off + rows, 8, cudaMemcpyDeviceToHost, s));
+    PCC_CUDA(cudaStreamSynchronize(s));
+    const int64_t total = h[0];
+    PCC_TRY(idx->keys64.reserve((size_t)std::max<int64_t>(total, 1) * sizeof(nkey_t)));
+    nkey_t *keys = idx->keys64.as<nkey_t>();
+    if (total > 0) {
+        seg_select_fill_kernel<<<nblocks(n, 128), 128, 0, s>>>(idx->grid(), seg, seg_off, d_off, params, keys);
+        PCC_LAUNCHED();
+        PCC_CUDA(cudaGetLastError());
+    }
+    return rows > 0 ? select_unpack_rows(idx, rows, k, d_off, keys, total, oi, od, s) : PCC_OK;
 }
 int pcc::sift_dog_segmented(pcc_index *idx, const uint32_t *seg, const float *values, const float *scales, int n_scales, float *out, cudaStream_t s) {
     const SiftScales sc = sift_scale_table(scales, n_scales);

@@ -91,6 +91,12 @@ class GridSearch:
     def getInputCloud(self):
         return self._cloud
 
+    def _adopt_input(self, cloud, mem, n: int):
+        """A batched entry rebuilt this index on `cloud` (n rows): self-queries (queries=None) now mean its rows.  n = 0 leaves the
+        index, and so this state, untouched."""
+        if n > 0:
+            self._cloud, self._mem, self._n_input = cloud, mem, n
+
     @property
     def size(self) -> int:
         return int(self._L.pcc_size(self._h))
@@ -378,6 +384,44 @@ def region_growing_rgb(neighbours, sqr_distances, rgba, distance_threshold: floa
     return labels, int(nc.value)
 
 
+def knn_batched(xyz, offsets, k: int, device: int = 0, workspace: "GridSearch | None" = None):
+    """RegionGrowingRGB::findPointNeighbours on every cluster [offsets[c], offsets[c+1]) of xyz in one pcc_knn_batched call: returns
+    (idx [n, k] int32, d2 [n, k] float32, k_eff int32 [n_clouds]); the rows of cluster c are GridSearch().setInputCloud(cluster, k_hint=k)
+    .nearestKSearch(None, k) of that cluster alone, bit for bit, with cluster-LOCAL indices.  numpy inputs go through PCC_HOST; a CUDA
+    tensor xyz keeps the call and the table on the device, on the current stream.  `workspace` is left indexing the concatenation."""
+    off = np.ascontiguousarray(np.asarray(offsets), np.int64)
+    n_clouds = off.shape[0] - 1
+    k_eff = np.zeros(max(n_clouds, 0) + 1, np.int32)
+    ws = workspace or GridSearch(device)
+    ptr, n, stride, mem, keep = _rows(xyz if _is_cuda(xyz) else np.asarray(xyz, np.float32))
+    idx, ip = ws._alloc(mem, (n, int(k)), np.int32)
+    d2, dp = ws._alloc(mem, (n, int(k)), np.float32)
+    check(ws._L.pcc_knn_batched(ws._h, ptr, n, stride, off.ctypes.data, n_clouds, int(k), ip, dp, k_eff.ctypes.data, mem, _stream(ws.device)))
+    ws._adopt_input(keep, mem, n)
+    return idx, d2, k_eff[:n_clouds]
+
+
+def region_growing_rgb_batched(xyz, rgb, offsets, k: int = 100, distance_threshold: float = 10.0, point_color_threshold: float = 6.0,
+                               region_color_threshold: float = 5.0, grow_neighbours: int = 30, min_size: int = 200, max_size: int = 2**31 - 1,
+                               device: int = 0, workspace: "GridSearch | None" = None):
+    """color_growing_segmentation (src/segmentation.cpp:161-216) on every cluster [offsets[c], offsets[c+1]) of xyz / rgb in one
+    pcc_region_growing_rgb_batched call: returns (labels int32 [n], n_clusters int64 [n_clouds]); labels of cluster c are cluster-LOCAL and
+    equal region_growing_rgb over knn_batched's table of that cluster alone.  rgb is uint8 [n, 3] (r, g, b).  The reference's "more than
+    10 points" test (src/segmentation.cpp:167) stays with the caller.  A CUDA tensor xyz runs the search on the device, on the current
+    stream; the grow runs on the host either way."""
+    off = np.ascontiguousarray(np.asarray(offsets), np.int64)
+    n_clouds = off.shape[0] - 1
+    rows, ptr, n, mem = _xyzrgb_rows(xyz, rgb)
+    labels = np.empty(max(n, 1), np.int32)
+    n_clusters = np.zeros(max(n_clouds, 0) + 1, np.int64)
+    ws = workspace or GridSearch(device)
+    check(ws._L.pcc_region_growing_rgb_batched(ws._h, ptr, n, 16, 12, off.ctypes.data, n_clouds, int(k), float(distance_threshold), float(point_color_threshold),
+                                               float(region_color_threshold), int(grow_neighbours), int(min_size), int(max_size), labels.ctypes.data,
+                                               n_clusters.ctypes.data, mem, _stream(ws.device)))
+    ws._adopt_input(rows, mem, n)
+    return labels[:n], n_clusters[:n_clouds]
+
+
 def descriptor_nn(ref, qry, dims: int | None = None, device: int = 0, workspace: "GridSearch | None" = None):
     """1-NN in descriptor space (matchRIFTFeaturesKnn, src/comparator.cpp:560-588): (index into ref or -1, squared distance).
     `dims` = leading floats of a row that take part (None = all columns; 3 = what PCL 1.7 compares for Histogram<32>, see search.h)."""
@@ -505,6 +549,18 @@ def _sift_rows(xyz, rgb):
     return rows
 
 
+def _xyzrgb_rows(xyz, rgb):
+    """_sift_rows in the memory kind of xyz: (rows, pointer, n, mem); a CUDA tensor xyz gets CUDA rows (PCC_DEVICE), else numpy (PCC_HOST)."""
+    if _is_cuda(xyz):
+        c = torch.as_tensor(np.asarray(rgb.cpu().numpy() if _is_cuda(rgb) else rgb).reshape(-1, 3).astype(np.int32), device=xyz.device)
+        rows = torch.empty((xyz.shape[0], 4), dtype=torch.float32, device=xyz.device)
+        rows[:, :3] = xyz[:, :3]
+        rows[:, 3] = ((c[:, 0] << 16) | (c[:, 1] << 8) | c[:, 2]).view(torch.float32)
+        return rows, rows.data_ptr(), rows.shape[0], DEVICE
+    rows = _sift_rows(xyz, rgb)
+    return rows, rows.ctypes.data, rows.shape[0], HOST
+
+
 def sift_keypoints(xyz, rgb, min_scale: float = 0.005, nr_octaves: int = 5, nr_scales_per_octave: int = 5, min_contrast: float = 0.001,
                    device: int = 0, stages: dict | None = None):
     """SIFTKeypoint<PointXYZRGB, PointWithScale>::compute as processSift configures it (src/comparator.cpp:449-465), one
@@ -558,18 +614,11 @@ def _sift_batched(xyz, rgb, offsets, snap_threshold, min_scale, nr_octaves, nr_s
     n_clouds = off.shape[0] - 1
     kp_off = np.zeros(max(n_clouds, 0) + 1, np.int64)
     want_snap = snap_threshold is not None
-    if _is_cuda(xyz):
-        dev = xyz.device
-        c = torch.as_tensor(np.asarray(rgb.cpu().numpy() if _is_cuda(rgb) else rgb).reshape(-1, 3).astype(np.int32), device=dev)
-        rows = torch.empty((xyz.shape[0], 4), dtype=torch.float32, device=dev)
-        rows[:, :3] = xyz[:, :3]
-        rows[:, 3] = ((c[:, 0] << 16) | (c[:, 1] << 8) | c[:, 2]).view(torch.float32)
-        ptr, n, mem = rows.data_ptr(), rows.shape[0], DEVICE
-        alloc = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)          # noqa: E731
+    rows, ptr, n, mem = _xyzrgb_rows(xyz, rgb)
+    if mem == DEVICE:
+        alloc = lambda shape, dt: torch.empty(shape, dtype=dt, device=xyz.device)   # noqa: E731
         f32, i32 = torch.float32, torch.int32
     else:
-        rows = _sift_rows(xyz, rgb)
-        ptr, n, mem = rows.ctypes.data, rows.shape[0], HOST
         alloc = lambda shape, dt: np.empty(shape, dt)                                 # noqa: E731
         f32, i32 = np.float32, np.int32
     L = _lib.lib()
